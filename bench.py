@@ -20,6 +20,8 @@ the same bytes from numpy and from torch on the GPU):
 host<->device copies inside the timed region.  Time = wall clock between barriers, max over ranks.
 The output of the timed steps is hashed (SHA-256) and compared with the oracle's golden
 (tests/golden/stream_sha.json, tools/make_golden_sha.py) and decoded with libbz2, outside the timed region.
+--dump-outputs DIR writes what the last timed step returned (rank 0's view) as DIR/<name>.npy, so that two builds can
+be compared output for output; see dump_outputs().
 """
 import argparse
 import bz2
@@ -99,6 +101,44 @@ def hbm_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT = 64_000_000     # bytes of all dumped arrays together
+DUMP_EDGE = 4096             # leading and trailing rows always dumped: stream header, last block, footer and stream CRC
+DUMP_SEED = 0x5EED00D0
+
+
+def sample_rows(n, n_max, seed=DUMP_SEED):
+    """Increasing int64 row numbers of a fixed, seeded sample of n rows: all of them when n <= n_max, else the first and
+    last DUMP_EDGE rows and one row at a seeded position in each of n_max equal strata.  They depend on n only, so two
+    runs that return the same arrays dump the same sample."""
+    if n <= n_max:
+        return np.arange(n, dtype=np.int64)
+    edges = np.arange(n_max + 1, dtype=np.int64) * n // n_max
+    pos = edges[:-1] + (np.random.default_rng(seed).random(n_max) * (edges[1:] - edges[:-1])).astype(np.int64)
+    return np.unique(np.concatenate([np.arange(DUMP_EDGE), pos, np.arange(n - DUMP_EDGE, n)]))
+
+
+def dump_outputs(out_dir, tables):
+    """tables: {name: (n_max, {column: 1-D integer array})}, the columns of a table of equal length.  Writes
+    out_dir/<name>_length.npy (float64, one element), <name>_positions.npy (float64, the rows of sample_rows(length,
+    n_max)) and <name>_<column>.npy for every column at those rows: float32 for bytes, float64 for wider integers
+    (exact below 2^53)."""
+    out = {}
+    for name, (n_max, cols) in tables.items():
+        n = len(next(iter(cols.values())))
+        pos = sample_rows(n, n_max)
+        out[name + "_length"] = np.array([n], np.float64)
+        out[name + "_positions"] = pos.astype(np.float64)
+        for col, a in cols.items():
+            a = np.asarray(a)
+            assert a.shape == (n,), (name, col, a.shape)
+            out["%s_%s" % (name, col)] = a[pos].astype(np.float32 if a.dtype == np.uint8 else np.float64)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_LIMIT, {k: a.nbytes for k, a in out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return out
 
 
 def golden(key):
@@ -231,7 +271,11 @@ def main():
     ap.add_argument("--cpu-sample-mb", type=float, default=4.0)
     ap.add_argument("--no-decode", action="store_true", help="skip the libbz2 round trip of the output")
     ap.add_argument("--stage-times", action="store_true", help="one extra diagnostic step with per-stage timers")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy "
+                    "(float32 / float64; long buffers as a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -401,6 +445,8 @@ def main():
     if rank != 0:
         dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stream": (4 << 20, {"bytes": stream})})
     sha = hashlib.sha256(stream.tobytes()).hexdigest()
     gkey = "%s:%d:%x:9" % (name, n, seed)
     g = golden(gkey)
@@ -554,6 +600,13 @@ def run_entries(args, rank, local_rank, world, dev, enc, b2, sharding, barrier, 
     if rank != 0:
         dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        # rank 0's archive volume and its entries, in the order of its share
+        dump_outputs(args.dump_outputs, {
+            "archive": (4 << 20, {"bytes": arch}),
+            "entries": (256 << 10, {col: np.array([getattr(x, f) for x in info], np.uint64) for col, f in
+                                    (("crc32", "crc32"), ("method", "zip_type"), ("compressed_size", "compressed_size"),
+                                     ("header_offset", "local_header_offset"))})})
     mbps = total_bytes * args.steps / 1e6 / wall
     # CPU baseline: the oracle's Zip.Create restatement on a bounded sample of the same entries, 1 thread
     import oracle_lib as orc
