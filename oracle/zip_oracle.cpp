@@ -153,21 +153,31 @@ int Check_Size(Zip_Create_Info &info, u64 value) {      // zip-create.adb:161-17
   return 0;
 }
 
+// Where Compress_Data takes the BZip2 stream of an entry from: encoded here (stream == nullptr), or given by the
+// caller (orc_zip_create_given), e.g. a stream the oracle cannot afford to encode in a test.
+struct Stream_Source { const u8 *stream = nullptr; u64 stream_len = 0; };
+
 // Zip.Compress.Compress_Data for a BZip2 single method (zip-compress.adb:60-237), input size known.
-void Compress_Data(Zip_Create_Info &info, const u8 *in, u64 input_size, u32 &CRC, u64 &output_size, u16 &zip_type) {
+void Compress_Data(Zip_Create_Info &info, const u8 *in, u64 input_size, const Stream_Source &src, u32 &CRC, u64 &output_size,
+                   u16 &zip_type) {
   const u64 idx_out = info.stream.index;                // :84
   Init(CRC);                                            // :150
   // BZip2_E (zip-compress-bzip2_e.adb:110-135): the CRC is updated by Read_Byte for every byte read
   // (:70-98); the encoder reads the whole input before the inefficiency test can fire on a flush.
-  std::vector<u8> comp((size_t)(input_size + input_size / 50 + 4096));
-  u64 comp_len = 0;
-  orc_encode_stream(in, input_size, info.level, (i64)input_size, 0, comp.data(), comp.size(), &comp_len, nullptr, 0, nullptr);
+  std::vector<u8> comp;
+  const u8 *comp_data = src.stream;
+  u64 comp_len = src.stream_len;
+  if (!comp_data) {
+    comp.resize((size_t)(input_size + input_size / 50 + 4096));
+    orc_encode_stream(in, input_size, info.level, (i64)input_size, 0, comp.data(), comp.size(), &comp_len, nullptr, 0, nullptr);
+    comp_data = comp.data();
+  }
   Update(CRC, in, input_size);
   // Write_Block raises Compression_inefficient as soon as output_size >= input_size (zip-compress.adb:468-490);
   // the running total reaches its maximum at the final flush, so the test is on the whole stream.
   bool compression_ok = !(comp_len >= input_size);
   if (compression_ok) {
-    info.stream.Write(comp.data(), comp_len);
+    info.stream.Write(comp_data, comp_len);
     output_size = comp_len;
     zip_type = 12;                                      // Compression_format_code.bzip2_code (:209)
   }
@@ -183,8 +193,8 @@ void Compress_Data(Zip_Create_Info &info, const u8 *in, u64 input_size, u32 &CRC
   }
 }
 
-int Add_Stream(Zip_Create_Info &info, const std::string &stream_name, const u8 *data, u64 size, u32 time, bool unicode,
-               bool read_only) {                        // zip-create.adb:194-297
+int Add_Stream(Zip_Create_Info &info, const std::string &stream_name, const u8 *data, u64 size, const Stream_Source &src, u32 time,
+               bool unicode, bool read_only) {                        // zip-create.adb:194-297
   std::string entry_name = stream_name;                 // Unixify (:180-192)
   for (char &c : entry_name) if (c == '\\') c = '/';
   info.contains.emplace_back();                         // Add_catalogue_entry (:103-134)
@@ -213,7 +223,7 @@ int Add_Stream(Zip_Create_Info &info, const std::string &stream_name, const u8 *
     fh_extra.tag = 1; fh_extra.size = (u16)(local_header_extension_short_length - 4);
     Write_Ext(info.stream, fh_extra, true);
   }
-  Compress_Data(info, data, size, shi.crc_32, shi.compressed_size, shi.zip_type);
+  Compress_Data(info, data, size, src, shi.crc_32, shi.compressed_size, shi.zip_type);
   const u64 mem2 = info.stream.index;
   info.stream.index = mem1;                             // rewrite with complete informations (:279-292)
   Write_Local(info.stream, shi, pol);
@@ -276,6 +286,26 @@ int Finish(Zip_Create_Info &info) {                     // zip-create.adb:645-75
   return 0;
 }
 
+int zip_create(int level, u32 n_entries, const u8 *in, const u64 *in_offsets, const u64 *sizes, const char *names,
+               const u32 *name_offsets, const u32 *dos_times, const u32 *flags, const u8 *streams, const u64 *stream_offsets,
+               const u64 *stream_lens, u8 *out, u64 out_cap, u64 *out_len, u16 *methods) {
+  Zip_Create_Info info;
+  info.level = level;
+  for (u32 i = 0; i < n_entries; i++) {
+    const std::string nm(names + name_offsets[i], names + name_offsets[i + 1]);
+    const u32 fl = flags ? flags[i] : 0;
+    Stream_Source src;
+    if (streams) { src.stream = streams + stream_offsets[i]; src.stream_len = stream_lens[i]; }
+    if (Add_Stream(info, nm, in + in_offsets[i], sizes[i], src, dos_times ? dos_times[i] : 16789u * 65536u, fl & 1u, fl & 2u)) return 3;
+    if (methods) methods[i] = info.contains.back().head.short_info.zip_type;
+  }
+  if (Finish(info)) return 3;
+  if (out_len) *out_len = info.stream.data.size();
+  if (info.stream.data.size() > out_cap) return 2;
+  if (out) memcpy(out, info.stream.data.data(), info.stream.data.size());
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -291,19 +321,17 @@ u32 orc_zip_crc32(const u8 *in, u64 n) {
 int orc_zip_create(int level, u32 n_entries, const u8 *in, const u64 *in_offsets, const u64 *sizes, const char *names,
                    const u32 *name_offsets, const u32 *dos_times, const u32 *flags, u8 *out, u64 out_cap, u64 *out_len,
                    u16 *methods) {
-  Zip_Create_Info info;
-  info.level = level;
-  for (u32 i = 0; i < n_entries; i++) {
-    const std::string nm(names + name_offsets[i], names + name_offsets[i + 1]);
-    const u32 fl = flags ? flags[i] : 0;
-    if (Add_Stream(info, nm, in + in_offsets[i], sizes[i], dos_times ? dos_times[i] : 16789u * 65536u, fl & 1u, fl & 2u)) return 3;
-    if (methods) methods[i] = info.contains.back().head.short_info.zip_type;
-  }
-  if (Finish(info)) return 3;
-  if (out_len) *out_len = info.stream.data.size();
-  if (info.stream.data.size() > out_cap) return 2;
-  if (out) memcpy(out, info.stream.data.data(), info.stream.data.size());
-  return 0;
+  return zip_create(level, n_entries, in, in_offsets, sizes, names, name_offsets, dos_times, flags, nullptr, nullptr, nullptr,
+                    out, out_cap, out_len, methods);
+}
+
+// The same archive with the BZip2 stream of entry i given as streams[stream_offsets[i] ..][0 .. stream_lens[i]) instead
+// of encoded here.  An entry with stream_lens[i] >= sizes[i] is stored, and its stream bytes are not read.
+int orc_zip_create_given(int level, u32 n_entries, const u8 *in, const u64 *in_offsets, const u64 *sizes, const char *names,
+                         const u32 *name_offsets, const u32 *dos_times, const u32 *flags, u8 *out, u64 out_cap, u64 *out_len,
+                         u16 *methods, const u8 *streams, const u64 *stream_offsets, const u64 *stream_lens) {
+  return zip_create(level, n_entries, in, in_offsets, sizes, names, name_offsets, dos_times, flags, streams, stream_offsets,
+                    stream_lens, out, out_cap, out_len, methods);
 }
 
 }  // extern "C"

@@ -182,3 +182,41 @@ def zip_create(entries, level=9, dos_times=None, flags=None):
                               out.ctypes.data_as(C.c_void_p), C.c_uint64(cap), C.byref(out_len), methods.ctypes.data_as(C.c_void_p))
     assert rc == 0, rc
     return out[:out_len.value].tobytes(), [int(m) for m in methods[:n]]
+
+
+def zip_create_given_flat(flat, offs, sizes, names, name_offs, streams, stream_offs, stream_lens, level=9, dos_times=None, flags=None):
+    """orc_zip_create_given on the flat arrays (no copy of the inputs): the archive of orc_zip_create with the BZip2
+    stream of entry i taken from streams[stream_offs[i]:][:stream_lens[i]] instead of encoded.  An entry whose
+    stream_len >= size is stored (pass stream_len = size for one known to be incompressible).
+    Returns (archive as a uint8 array, [method per entry])."""
+    n = int(sizes.size)
+    sizes = np.ascontiguousarray(sizes, np.uint64)
+    offs = np.ascontiguousarray(offs, np.uint64)
+    so = np.ascontiguousarray(stream_offs, np.uint64)
+    sl = np.ascontiguousarray(stream_lens, np.uint64)
+    st = _u8(streams) if streams is not None and len(streams) else np.zeros(1, np.uint8)
+    cap = int(sizes.sum()) + int(name_offs[-1]) * 2 + n * 124 + 200
+    out = np.empty(cap, np.uint8)
+    out_len = C.c_uint64(0)
+    methods = np.zeros(max(n, 1), np.uint16)
+    t = None if dos_times is None else np.ascontiguousarray(dos_times, np.uint32)
+    f = None if flags is None else np.ascontiguousarray(flags, np.uint32)
+    rc = lib().orc_zip_create_given(level, C.c_uint32(n), flat.ctypes.data_as(C.c_void_p), offs.ctypes.data_as(C.c_void_p),
+                                    sizes.ctypes.data_as(C.c_void_p), C.c_char_p(names), name_offs.ctypes.data_as(C.c_void_p),
+                                    None if t is None else t.ctypes.data_as(C.c_void_p), None if f is None else f.ctypes.data_as(C.c_void_p),
+                                    out.ctypes.data_as(C.c_void_p), C.c_uint64(cap), C.byref(out_len), methods.ctypes.data_as(C.c_void_p),
+                                    st.ctypes.data_as(C.c_void_p), so.ctypes.data_as(C.c_void_p), sl.ctypes.data_as(C.c_void_p))
+    assert rc == 0, rc
+    return out[:out_len.value], [int(m) for m in methods[:n]]
+
+
+def zip_create_given(entries, streams, level=9, dos_times=None, flags=None):
+    """entries: list of (name, bytes-like); streams: one bytes-like per entry (its BZip2 stream; for an entry to be
+    stored, any object whose len() is >= the entry's size).  Returns (archive bytes, [method per entry])."""
+    flat, offs, sizes, names, name_offs = pack_entries(entries)
+    lens = np.array([len(s) for s in streams], np.uint64)
+    given = [b"" if int(l) >= int(sz) else bytes(s) for s, l, sz in zip(streams, lens, sizes)]
+    so = np.zeros(len(given), np.uint64)
+    so[1:] = np.cumsum([len(g) for g in given])[:-1] if given else []
+    arc, methods = zip_create_given_flat(flat, offs, sizes, names, name_offs, b"".join(given), so, lens, level, dos_times, flags)
+    return arc.tobytes(), methods

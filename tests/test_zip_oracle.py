@@ -6,6 +6,7 @@ import zipfile
 import zlib
 
 import numpy as np
+import pytest
 
 import datagen
 import oracle_lib as orc
@@ -100,3 +101,16 @@ def test_pin_script_reads_an_entry_payload():
     method, payload = pin.payload_of_single_entry(arc)
     assert method == 12 == methods[0]
     assert payload == orc.encode_stream(data, 9, len(data))
+
+
+@pytest.mark.parametrize("level", [1, 4, 9])
+def test_given_streams_give_the_same_archive(level):
+    """orc_zip_create_given with each entry's stream from orc_encode_stream is orc_zip_create, byte for byte:
+    the same Add_Stream / Store decision / header rewrite / Finish, only the stream source differs."""
+    ents = _entries()
+    streams = [orc.encode_stream(d, level, len(d)) for _, d in ents]
+    t = [16789 * 65536 + 3 * i for i in range(len(ents))]
+    fl = [1, 0, 2, 0, 3, 0]
+    ref, methods = orc.zip_create(ents, level, dos_times=t, flags=fl)
+    got, methods_given = orc.zip_create_given(ents, streams, level, dos_times=t, flags=fl)
+    assert got == ref and methods_given == methods

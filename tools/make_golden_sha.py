@@ -28,6 +28,7 @@ DEFAULT = [
     "markov:%d:5eed0001:9" % (2048 * MiB),      # one stream over 2 / 4 / 8 GPUs, 1 GiB per GPU
     "markov:%d:5eed0001:9" % (4096 * MiB),
     "markov:%d:5eed0001:9" % (8192 * MiB),
+    "mixed:%d:5eed0004:9" % (4352 * MiB),       # one stream past 2^32 bytes (tests/test_gpu_past_4gib.py)
 ]
 
 
