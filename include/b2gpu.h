@@ -138,6 +138,38 @@ B2_API int b2_shard_finish(b2_encoder *enc, uint64_t bit_offset, uint32_t crc_in
 B2_API int b2_encode_stream_multi(b2_encoder **encs, int n_encs, const uint8_t *in, uint64_t n, int64_t size_hint,
                                   uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 
+/* ---- One stream fed in pieces (the streaming shape of Encode: Read_Byte / More_Bytes / Write_Byte) ------------
+ * Incremental Encode (option, size_hint): input in pieces, finished output in pieces.
+ * The concatenation of every out of b2_stream_write and b2_stream_end is byte-identical to what
+ * b2_encode_stream gives for the concatenated input and the same size_hint.
+ *   - One open stream per handle.  While it is open, every other call that uses the handle's device buffers
+ *     (encode, batch, zip, shard, verify, zip_crc32, dbg) returns B2_ERR_ARGUMENT; b2_stream_*, b2_set_*,
+ *     b2_get_*, b2_reset_stats and b2_destroy are allowed.
+ *   - The handle holds the bytes not yet encoded on the device, from the start of the next chunk.  When
+ *     window_bytes + b2_shard_margin (level) of them are held, it encodes the chunks that start in the first
+ *     window_bytes (a shard of the stream whose bit offset and CRC are known) and keeps the rest.  Device input
+ *     memory is at most 2 x (window_bytes + b2_shard_margin + 256) bytes, whatever the stream length and write sizes.
+ *     window_bytes: 0 = 512 MiB; below 1 MiB is B2_ERR_ARGUMENT.
+ *   - `in` is host memory (pinned memory lets the upload run under the encode of the window before); the caller
+ *     may reuse it as soon as the write returns.  `out` receives every byte that is final; the last partial byte
+ *     is held back until the next window's bits or the footer complete it.
+ *   - out_cap < b2_stream_bound (enc, n) returns B2_ERR_OUTPUT_TOO_SMALL before any input is taken: the stream is
+ *     unchanged and the call can be repeated.  Any other error, B2_ERR_ABORTED included, closes the stream; the
+ *     handle stays usable.
+ *   - b2_set_progress fires after every device batch with the stream bytes encoded so far and size_hint (or, when
+ *     it is unknown, that plus the bytes held); a non-zero return ends the write with B2_ERR_ABORTED.
+ *   - b2_stats counts one stream; b2_get_trace after b2_stream_end gives every chunk with stream offsets. */
+B2_API int b2_stream_begin(b2_encoder *enc, int64_t size_hint, uint64_t window_bytes);
+/* An out_cap that always suffices for a write of n bytes (b2_stream_end: n = 0) in the stream's current state. */
+B2_API uint64_t b2_stream_bound(b2_encoder *enc, uint64_t n);
+B2_API int b2_stream_write(b2_encoder *enc, const uint8_t *in, uint64_t n,
+                           uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+/* Encodes what is held as the last window and writes the footer ("BZh<level>" and the footer alone for an empty
+ * stream); closes the stream. */
+B2_API int b2_stream_end(b2_encoder *enc, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+/* Closes the open stream, if any, discarding what it holds. */
+B2_API int b2_stream_abort(b2_encoder *enc);
+
 /* ---- Archive side: batched Zip.Create for BZip2 entries ------------------------------------------
  * One call = Create_Archive, Add_Stream for every entry, Finish (zip-create.adb:194-297, :645-756)
  * with Compress_Method = BZip2_1/2/3 (the level of `enc`), no password.  The bytes written to `out`

@@ -62,7 +62,8 @@ EXPORTS = ["b2_create", "b2_destroy", "b2_bound", "b2_encode_stream", "b2_encode
            "b2_set_timing", "b2_get_stats", "b2_reset_stats", "b2_dbg_block", "b2_get_trace", "b2_get_segments",
            "b2_zip_bound", "b2_zip_create", "b2_zip_crc32",
            "b2_shard_margin", "b2_shard_plan", "b2_shard_open", "b2_shard_cut", "b2_shard_encode", "b2_shard_resolve",
-           "b2_shard_finish", "b2_encode_stream_multi", "b2_set_progress", "b2_verify_stream"]
+           "b2_shard_finish", "b2_encode_stream_multi", "b2_set_progress", "b2_verify_stream",
+           "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort"]
 
 _lib = None
 
@@ -109,6 +110,12 @@ def lib():
         _lib.b2_shard_resolve.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         _lib.b2_shard_finish.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_int, C.c_uint64,
                                          C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint8), C.POINTER(C.c_uint8)]
+        _lib.b2_stream_begin.argtypes = [C.c_void_p, C.c_int64, C.c_uint64]
+        _lib.b2_stream_bound.restype = C.c_uint64
+        _lib.b2_stream_bound.argtypes = [C.c_void_p, C.c_uint64]
+        _lib.b2_stream_write.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        _lib.b2_stream_end.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        _lib.b2_stream_abort.argtypes = [C.c_void_p]
         _lib.b2_encode_stream_multi.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_int64, C.c_void_p, C.c_uint64,
                                                 C.POINTER(C.c_uint64)]
     return _lib
@@ -269,6 +276,13 @@ class Encoder:
                                      C.byref(fb), C.byref(lb)))
         return off.value, ln.value, fb.value, lb.value
 
+    # -- one stream fed in pieces (b2_stream_*) --------------------------------------------------
+    def stream(self, size_hint=unknown_size, window=0):
+        """Opens the handle's stream: `Stream.write(data)` and `Stream.end()` return the bytes that are final so
+        far; together they are `encode(all data, size_hint)`.  window: bytes per device window (0 = 512 MiB)."""
+        _check(lib().b2_stream_begin(self._h, int(size_hint), int(window)))
+        return Stream(self)
+
     # -- generic shape of the reference: Read_Byte / More_Bytes / Write_Byte --------------------
     def encode_callbacks(self, read_byte, more_bytes, write_byte, size_hint=unknown_size):
         buf = bytearray()
@@ -345,6 +359,42 @@ class Encoder:
         return dict(rle=rle[:info.n_rle].copy(), bwt=bwt[:info.n_rle].copy(), mtf=mtf[:info.n_mtf].copy(),
                     sel=sel[:info.n_sel].copy(), lens=lens.reshape(6, 258).copy(),
                     bits=bits[:(info.bits + 7) // 8].copy(), info=info)
+
+
+class Stream:
+    """The open stream of an Encoder (Encoder.stream).  As a context manager it aborts the stream when the block
+    raises, so that the handle can encode again."""
+
+    def __init__(self, enc):
+        self.enc = enc
+
+    def _run(self, fn, n, *args):
+        cap = int(lib().b2_stream_bound(self.enc._h, n))
+        out = np.empty(cap, dtype=np.uint8)
+        out_len = C.c_uint64(0)
+        _check(fn(self.enc._h, *args, out.ctypes.data, cap, C.byref(out_len)))
+        return out[:out_len.value].tobytes()
+
+    def write(self, data):
+        a = _u8(data)
+        return self._run(lib().b2_stream_write, a.size, a.ctypes.data if a.size else None, a.size)
+
+    def write_ptr(self, in_ptr, n):
+        """Host pointer (e.g. a pinned torch tensor)."""
+        return self._run(lib().b2_stream_write, n, in_ptr, n)
+
+    def end(self):
+        return self._run(lib().b2_stream_end, 0)
+
+    def abort(self):
+        _check(lib().b2_stream_abort(self.enc._h))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, *a):
+        if exc_type is not None:
+            self.abort()
 
 
 def shard_plan(n, n_shards, level=block_900k, stagger_permille=-1):

@@ -40,6 +40,8 @@ void b2_set_error(const char *file, int line, const char *msg) {
 }
 #define B2_FAIL(code, msg) do { b2_set_error(__FILE__, __LINE__, msg); return code; } while (0)
 #define B2_TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
+// calls that use the handle's device buffers are refused while b2_stream_* owns them
+#define B2_NO_STREAM(e) do { if ((e)->stream.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is open on this handle (b2_stream_begin)"); } while (0)
 
 namespace {
 
@@ -128,21 +130,42 @@ struct Workspace {
 
 }  // namespace
 
-// One stream spread over several handles (b2_shard_*): what this handle keeps between the calls.
+// One stream spread over several handles (b2_shard_*), or one window of a stream fed in pieces (b2_stream_*):
+// what this handle keeps between the calls.
 struct ShardCand { u32 arena; u32 blocks; u64 word_off; u64 nbits; u32 fold; u32 kept; };
 struct ShardState {
   bool open = false, cut = false, encoded = false;
+  bool last = false;                   // the shard ends the stream: its chain walks to the end of its bytes, it writes the footer
   const u8 *d_in = nullptr;            // the shard's bytes on the device: stream bytes [base, base + n_local)
-  u64 base = 0, n_local = 0, stream_n = 0, own_end = 0, entry = 0, handoff = 0;
+  u64 base = 0, n_local = 0, own_end = 0, entry = 0, handoff = 0;
   i64 hint = -1;
   std::vector<DevBuf<u32> *> arenas;   // candidate bitstreams that may still win, one arena per batch (kept across calls)
   std::vector<ShardCand> cands;        // [chunk][tactic]
   std::vector<int> n_tactics;
 };
 
+// One stream fed in pieces (b2_stream_*).  Every window is a shard of the stream on this handle (DESIGN.md §6b).
+struct StreamState {
+  bool open = false;
+  i64 hint = -1;
+  u64 window = 0, margin = 0;          // W, and M = b2_shard_margin (level)
+  u8 *buf[2] = {nullptr, nullptr};     // two window buffers of W + M + 256 bytes (kept across streams of the same W)
+  u64 buf_bytes = 0;
+  int cur = 0;                         // buf[cur] holds the stream bytes [base, base + held), not encoded yet
+  u64 base = 0, held = 0;
+  u64 bit = 32;                        // stream bit offset where the next window's first block starts
+  u32 crc = 0;                         // combined CRC before it
+  u64 out_end = 0;                     // stream bytes whose final value has been written to an `out`
+  u8 tail = 0;                         // the bits of byte out_end so far (the partial byte held back)
+  std::vector<b2_chunk_trace> trace;   // every chunk of the stream so far, stream offsets
+};
+
 struct b2_encoder {
   int level = 9, device = 0;
   ShardState shard;
+  StreamState stream;
+  cudaStream_t cst = nullptr;           // uploads of b2_stream_write, overlapping the encode of the window before
+  cudaEvent_t ev_up = nullptr;          // recorded on cst after every upload
   b2_progress_fn progress = nullptr;    // called on the calling thread between batches; non-zero return aborts
   void *progress_user = nullptr;
   cudaStream_t st = nullptr;            // stream of the stream-level work (cut, segment, copies, footer)
@@ -948,6 +971,8 @@ int b2_create(int level, int device, b2_encoder **out) {
   auto init = [&]() -> int {
     B2_CUDA_CHECK(cudaStreamCreateWithFlags(&e->st, cudaStreamNonBlocking));
     B2_CUDA_CHECK(cudaStreamCreateWithFlags(&e->st2, cudaStreamNonBlocking));
+    B2_CUDA_CHECK(cudaStreamCreateWithFlags(&e->cst, cudaStreamNonBlocking));
+    B2_CUDA_CHECK(cudaEventCreateWithFlags(&e->ev_up, cudaEventDisableTiming));
     B2_CUDA_CHECK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
     B2_CUDA_CHECK(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
     B2_CUDA_CHECK(cudaEventCreate(&e->ev[0])); B2_CUDA_CHECK(cudaEventCreate(&e->ev[1]));
@@ -985,6 +1010,9 @@ void b2_destroy(b2_encoder *e) {
   if (!e) return;
   cudaSetDevice(e->device);
   if (e->st) cudaStreamSynchronize(e->st);
+  if (e->cst) { cudaStreamSynchronize(e->cst); cudaStreamDestroy(e->cst); }
+  if (e->ev_up) cudaEventDestroy(e->ev_up);
+  for (int i = 0; i < 2; i++) if (e->stream.buf[i]) cudaFree(e->stream.buf[i]);
   for (auto *w : e->ws) { if (w->st) cudaStreamSynchronize(w->st); w->release(); delete w; }
   e->ws.clear();
   e->d_ct.release(); e->d_T.release(); e->d_in.release(); e->d_out.release(); e->d_chunks.release();
@@ -1007,6 +1035,7 @@ void b2_destroy(b2_encoder *e) {
 int b2_encode_stream_device(b2_encoder *e, const uint8_t *d_in, uint64_t n, int64_t size_hint,
                             uint8_t *d_out, uint64_t out_cap, uint64_t *out_len) {
   if (!e || !out_len || (n && !d_in)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   u64 len = 0;
   if (e->timing) cudaEventRecord(e->ev_call[0], e->st);
@@ -1023,6 +1052,7 @@ int b2_encode_stream_device(b2_encoder *e, const uint8_t *d_in, uint64_t n, int6
 int b2_encode_stream(b2_encoder *e, const uint8_t *in, uint64_t n, int64_t size_hint,
                      uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
   if (!e || !out_len || (n && !in)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   B2_TRY(e->d_in.ensure(n + 256));
   if (e->timing) cudaEventRecord(e->ev_call[0], e->st);
@@ -1049,6 +1079,7 @@ int b2_encode_batch(b2_encoder *e, uint32_t n_entries, const uint8_t *in, const 
                     const uint64_t *sizes, const int64_t *size_hints, uint8_t *out, uint64_t out_cap,
                     uint64_t *out_offsets, uint64_t *out_lens) {
   if (!e || (n_entries && (!in_offsets || !sizes || !out_offsets || !out_lens))) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   u64 total_in = 0;
   for (u32 i = 0; i < n_entries; i++) total_in = std::max<u64>(total_in, in_offsets[i] + sizes[i]);
@@ -1113,40 +1144,30 @@ int b2_shard_plan(uint64_t n, int n_shards, int level, int stagger_permille, uin
   return 0;
 }
 
-int b2_shard_resolve(const b2_shard_link *links, int n_shards, uint64_t *bit_offsets, uint32_t *crcs) {
-  if (!links || !bit_offsets || !crcs || n_shards < 1) return B2_ERR_ARGUMENT;
-  bit_offsets[0] = 32; crcs[0] = 0;                  // behind "BZh<level>" (:1384-1391)
-  for (int r = 0; r < n_shards; r++) {
-    const u32 ph = (u32)(bit_offsets[r] & 7);
-    bit_offsets[r + 1] = bit_offsets[r] + links[r].total_bits[ph];
-    const u32 k = links[r].crc_rot[ph] & 31u, c = crcs[r];
-    crcs[r + 1] = (k ? ((c << k) | (c >> (32 - k))) : c) ^ links[r].crc_fold[ph];
-  }
-  return 0;
+}  // extern "C"
+
+namespace {
+// What a shard does to the bit offset and the combined CRC, given the incoming ones (:990, :1319-1345).
+void link_step(const b2_shard_link &l, u64 &bit, u32 &crc) {
+  const u32 ph = (u32)(bit & 7);
+  const u32 k = l.crc_rot[ph] & 31u;
+  crc = (k ? ((crc << k) | (crc >> (32 - k))) : crc) ^ l.crc_fold[ph];
+  bit += l.total_bits[ph];
 }
 
-int b2_shard_open(b2_encoder *e, const uint8_t *in, int in_is_device, uint64_t base, uint64_t n_local,
-                  uint64_t stream_size, int64_t size_hint, uint64_t own_end) {
-  if (!e || (n_local && !in) || base + n_local > stream_size || own_end > stream_size || own_end < base) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
-  B2_CUDA_CHECK(cudaSetDevice(e->device));
+// The four steps of a shard on this handle, for b2_shard_* and for the windows of b2_stream_*.
+// d_in: the stream bytes [base, base + n_local) on the device, followed by 128 zero bytes.
+int shard_load(b2_encoder *e, const u8 *d_in, u64 base, u64 n_local, u64 own_end, bool last, i64 size_hint) {
   B2_CUDA_CHECK(cudaStreamSynchronize(e->st2));
   ShardState &sh = e->shard;
   sh.open = sh.cut = sh.encoded = false;
-  sh.base = base; sh.n_local = n_local; sh.stream_n = stream_size; sh.hint = size_hint; sh.own_end = own_end;
-  if (e->timing) cudaEventRecord(e->ev_call[0], e->st);
-  if (in_is_device) sh.d_in = in;
-  else {
-    B2_TRY(e->d_in.ensure(n_local + 256));
-    if (n_local) B2_CUDA_CHECK(cudaMemcpyAsync(e->d_in.p, in, n_local, cudaMemcpyHostToDevice, e->st));
-    B2_CUDA_CHECK(cudaMemsetAsync(e->d_in.p + n_local, 0, 128, e->st));
-    sh.d_in = e->d_in.p;
-  }
+  sh.d_in = d_in; sh.base = base; sh.n_local = n_local; sh.own_end = own_end; sh.last = last; sh.hint = size_hint;
   // the scans of the cutting do not depend on where the first chunk starts: they run while the shards
   // before this one are still cutting
   const size_t ct = (size_t)(n_local / 2048 + 2);
   B2_TRY(e->d_cut_first.ensure(ct)); B2_TRY(e->d_cut_last.ensure(ct)); B2_TRY(e->d_cut_tsum.ensure(ct));
   B2_TRY(e->d_cut_carry.ensure(ct)); B2_TRY(e->d_cut_tincl.ensure(ct));
-        B2_TRY(e->d_cut_gs.ensure(ct * 128)); B2_TRY(e->d_cut_gm.ensure(ct * 128));
+  B2_TRY(e->d_cut_gs.ensure(ct * 128)); B2_TRY(e->d_cut_gm.ensure(ct * 128));
   B2CutWork cw{e->d_cut_first.p, e->d_cut_last.p, e->d_cut_tsum.p, e->d_cut_carry.p, e->d_cut_tincl.p, e->d_cut_gs.p, e->d_cut_gm.p};
   B2_TRY(b2k_cut_scans(e->st, sh.d_in, n_local, &cw));
   e->launches_other += 4;
@@ -1154,12 +1175,8 @@ int b2_shard_open(b2_encoder *e, const uint8_t *in, int in_is_device, uint64_t b
   return 0;
 }
 
-int b2_shard_cut(b2_encoder *e, uint64_t entry, uint64_t *handoff) {
-  if (!e || !handoff) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+int shard_cut(b2_encoder *e, u64 entry, u64 *handoff) {
   ShardState &sh = e->shard;
-  if (!sh.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_cut without b2_shard_open");
-  if (entry < sh.base || entry > sh.base + sh.n_local) B2_FAIL(B2_ERR_ARGUMENT, "entry outside the shard's bytes");
-  B2_CUDA_CHECK(cudaSetDevice(e->device));
   cudaStream_t st = e->st;
   const int level = e->level;
   e->trace.clear(); e->chunks.clear(); e->nseg.clear(); e->seg.clear();
@@ -1176,8 +1193,7 @@ int b2_shard_cut(b2_encoder *e, uint64_t entry, uint64_t *handoff) {
     B2_CUDA_CHECK(cudaMemsetAsync(e->d_nseg.p, 0xFE, (size_t)max_chunks * 2 * sizeof(u32), st));
   }
   // the last shard walks to the end of the stream; the others stop at the first chunk that belongs to the next one
-  const bool last = sh.own_end >= sh.stream_n;
-  const u64 stop = last ? sh.n_local : sh.own_end - sh.base;
+  const u64 stop = sh.last ? sh.n_local : sh.own_end - sh.base;
   B2_TRY(b2k_cut_chain(st, sh.d_in, sh.n_local, sh.hint, level, win_lo, win_hi, e->d_chunks.p, e->d_scalars.p, max_chunks, &cw,
                        follow ? e->d_scalars.p + 12 : nullptr, follow ? e->ev_fork : nullptr, sh.base, entry - sh.base, stop));
   e->launches_other += 1;
@@ -1202,15 +1218,11 @@ int b2_shard_cut(b2_encoder *e, uint64_t entry, uint64_t *handoff) {
   return 0;
 }
 
-int b2_shard_encode(b2_encoder *e, b2_shard_link *link) {
-  if (!e || !link) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+int shard_encode(b2_encoder *e, b2_shard_link *link) {
   ShardState &sh = e->shard;
-  if (!sh.cut) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_encode without b2_shard_cut");
-  B2_CUDA_CHECK(cudaSetDevice(e->device));
   const u32 nc = (u32)e->chunks.size();
   std::vector<StreamDesc> streams(1);
   streams[0] = StreamDesc{0, sh.n_local, sh.hint, 0, 0, 0, nc};
-  e->stats.streams++; e->stats.input_bytes += sh.handoff - sh.entry;
   std::vector<u32> chunk_stream(nc, 0u);
   const bool followed = e->level == 9 && e->timing < 2;
   B2_TRY(encode_chunks(e, sh.d_in, streams, chunk_stream, followed, &sh));
@@ -1232,14 +1244,11 @@ int b2_shard_encode(b2_encoder *e, b2_shard_link *link) {
   return 0;
 }
 
-int b2_shard_finish(b2_encoder *e, uint64_t bit_offset, uint32_t crc_in, uint8_t *out, int out_is_device, uint64_t out_cap,
-                    uint64_t *out_byte_offset, uint64_t *out_len, uint8_t *first_byte, uint8_t *last_byte) {
-  if (!e || !out_len || !out_byte_offset) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+int shard_finish(b2_encoder *e, u64 bit_offset, u32 crc_in, u8 *out, int out_is_device, u64 out_cap,
+                 u64 *out_byte_offset, u64 *out_len, u8 *first_byte, u8 *last_byte) {
   ShardState &sh = e->shard;
-  if (!sh.encoded) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_finish without b2_shard_encode");
-  B2_CUDA_CHECK(cudaSetDevice(e->device));
   cudaStream_t st = e->st;
-  const bool first = sh.base == 0 && sh.entry == 0, last = sh.own_end >= sh.stream_n;
+  const bool first = sh.base == 0 && sh.entry == 0, last = sh.last;
   if (first && bit_offset != 32) B2_FAIL(B2_ERR_ARGUMENT, "the first shard starts behind the 32-bit stream header");
   const u64 byte0 = first ? 0 : bit_offset >> 3;         // first byte of the stream this shard touches
   const u64 lbit0 = bit_offset - 8 * byte0;              // its bits start here in its piece
@@ -1301,6 +1310,234 @@ int b2_shard_finish(b2_encoder *e, uint64_t bit_offset, uint32_t crc_in, uint8_t
   sh.encoded = false; sh.cut = false; sh.open = false;
   return 0;
 }
+}  // namespace
+
+extern "C" {
+
+int b2_shard_resolve(const b2_shard_link *links, int n_shards, uint64_t *bit_offsets, uint32_t *crcs) {
+  if (!links || !bit_offsets || !crcs || n_shards < 1) return B2_ERR_ARGUMENT;
+  bit_offsets[0] = 32; crcs[0] = 0;                  // behind "BZh<level>" (:1384-1391)
+  for (int r = 0; r < n_shards; r++) {
+    u64 bit = bit_offsets[r]; u32 crc = crcs[r];
+    link_step(links[r], bit, crc);
+    bit_offsets[r + 1] = bit; crcs[r + 1] = crc;
+  }
+  return 0;
+}
+
+int b2_shard_open(b2_encoder *e, const uint8_t *in, int in_is_device, uint64_t base, uint64_t n_local,
+                  uint64_t stream_size, int64_t size_hint, uint64_t own_end) {
+  if (!e || (n_local && !in) || base + n_local > stream_size || own_end > stream_size || own_end < base) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  B2_CUDA_CHECK(cudaStreamSynchronize(e->st2));
+  e->shard.open = e->shard.cut = e->shard.encoded = false;
+  if (e->timing) cudaEventRecord(e->ev_call[0], e->st);
+  const u8 *d_in = in;
+  if (!in_is_device) {
+    B2_TRY(e->d_in.ensure(n_local + 256));
+    if (n_local) B2_CUDA_CHECK(cudaMemcpyAsync(e->d_in.p, in, n_local, cudaMemcpyHostToDevice, e->st));
+    B2_CUDA_CHECK(cudaMemsetAsync(e->d_in.p + n_local, 0, 128, e->st));
+    d_in = e->d_in.p;
+  }
+  return shard_load(e, d_in, base, n_local, own_end, own_end >= stream_size, size_hint);
+}
+
+int b2_shard_cut(b2_encoder *e, uint64_t entry, uint64_t *handoff) {
+  if (!e || !handoff) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
+  ShardState &sh = e->shard;
+  if (!sh.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_cut without b2_shard_open");
+  if (entry < sh.base || entry > sh.base + sh.n_local) B2_FAIL(B2_ERR_ARGUMENT, "entry outside the shard's bytes");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  return shard_cut(e, entry, handoff);
+}
+
+int b2_shard_encode(b2_encoder *e, b2_shard_link *link) {
+  if (!e || !link) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
+  ShardState &sh = e->shard;
+  if (!sh.cut) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_encode without b2_shard_cut");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  e->stats.streams++; e->stats.input_bytes += sh.handoff - sh.entry;
+  return shard_encode(e, link);
+}
+
+int b2_shard_finish(b2_encoder *e, uint64_t bit_offset, uint32_t crc_in, uint8_t *out, int out_is_device, uint64_t out_cap,
+                    uint64_t *out_byte_offset, uint64_t *out_len, uint8_t *first_byte, uint8_t *last_byte) {
+  if (!e || !out_len || !out_byte_offset) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
+  if (!e->shard.encoded) B2_FAIL(B2_ERR_ARGUMENT, "b2_shard_finish without b2_shard_encode");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  return shard_finish(e, bit_offset, crc_in, out, out_is_device, out_cap, out_byte_offset, out_len, first_byte, last_byte);
+}
+
+}  // extern "C"
+
+// ---- one stream fed in pieces (b2_stream_*, DESIGN.md §6b) ---------------------------------------------------------
+// Every window is a shard of the stream on this handle whose incoming bit offset and CRC are already known: it owns
+// the chunks that start before base + W, and a chunk that starts there ends before base + W + M, so it sees the bytes
+// of a one-shot encode.  The bytes from the next chunk start on move to the head of the other window buffer.
+namespace {
+struct ProgressShim { b2_progress_fn fn; void *user; u64 done0, total; };
+int progress_shim(void *u, u64 done, u64 total) {
+  (void)total;
+  const ProgressShim *p = (const ProgressShim *)u;
+  return p->fn(p->user, p->done0 + done, p->total);
+}
+
+void stream_close(b2_encoder *e) {
+  cudaStreamSynchronize(e->cst);                       // no upload may read the caller's `in` after the call returns
+  e->stream.open = false;
+  e->shard.open = e->shard.cut = e->shard.encoded = false;
+}
+
+int stream_upload(b2_encoder *e, int b, u64 at, const u8 *in, u64 k) {
+  if (!k) return 0;
+  B2_CUDA_CHECK(cudaMemcpyAsync(e->stream.buf[b] + at, in, k, cudaMemcpyHostToDevice, e->cst));
+  B2_CUDA_CHECK(cudaEventRecord(e->ev_up, e->cst));
+  return 0;
+}
+
+// Encodes the held bytes as one window and writes its finished bytes to out[stream byte - out0].  A window that is
+// not the last moves the bytes behind it to the other buffer and, before its blocks are encoded, enqueues the upload
+// of what follows them from in[*taken, n), so that the copy runs under the encode.
+int stream_window(b2_encoder *e, bool last, const u8 *in, u64 n, u64 *taken, u8 *out, u64 out_cap, u64 out0) {
+  StreamState &S = e->stream;
+  cudaStream_t st = e->st;
+  u8 *d = S.buf[S.cur];
+  if (e->timing) cudaEventRecord(e->ev_call[0], st);
+  B2_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_up, 0));
+  B2_CUDA_CHECK(cudaMemsetAsync(d + S.held, 0, 256, st));
+  B2_TRY(shard_load(e, d, S.base, S.held, last ? S.base + S.held : S.base + S.window, last, S.hint));
+  u64 handoff = 0;
+  B2_TRY(shard_cut(e, S.base, &handoff));
+  const int nxt = S.cur ^ 1;
+  u64 next_held = 0;
+  if (!last) {
+    const u64 carry = S.base + S.held - handoff;
+    B2_CUDA_CHECK(cudaMemcpyAsync(S.buf[nxt], d + (handoff - S.base), carry, cudaMemcpyDeviceToDevice, e->cst));
+    const u64 k = std::min<u64>(S.window + S.margin - carry, n - *taken);
+    B2_CUDA_CHECK(cudaEventRecord(e->ev_up, e->cst));
+    B2_TRY(stream_upload(e, nxt, carry, in + *taken, k));
+    *taken += k;
+    next_held = carry + k;
+  }
+  b2_shard_link link;
+  {
+    ProgressShim ps{e->progress, e->progress_user, S.base, S.hint >= 0 ? (u64)S.hint : S.base + S.held};
+    if (ps.fn) { e->progress = progress_shim; e->progress_user = &ps; }
+    const int rc = shard_encode(e, &link);
+    e->progress = ps.fn; e->progress_user = ps.user;
+    B2_TRY(rc);
+  }
+  u64 bit = S.bit;
+  u32 crc = S.crc;
+  link_step(link, bit, crc);
+  const u64 piece = S.base == 0 ? 0 : S.bit >> 3;      // where the window's bytes start in the stream
+  u64 off = 0, len = 0;
+  B2_TRY(shard_finish(e, S.bit, S.crc, out + (piece - out0), 0, out_cap - (piece - out0), &off, &len, nullptr, nullptr));
+  if (off != piece) B2_FAIL(B2_ERR_INTERNAL, "window piece misplaced");
+  if (len) out[piece - out0] |= S.tail;                // the byte held back from the window before
+  S.trace.insert(S.trace.end(), e->trace.begin(), e->trace.end());
+  e->stats.input_bytes += (last ? S.base + S.held : handoff) - S.base;
+  S.bit = bit; S.crc = crc;
+  if (last) { S.out_end = piece + len; S.tail = 0; S.held = 0; return 0; }
+  S.out_end = bit >> 3;
+  S.tail = (bit & 7) ? out[S.out_end - out0] : 0;
+  S.cur = nxt; S.base = handoff; S.held = next_held;
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+uint64_t b2_stream_bound(b2_encoder *e, uint64_t n) {
+  const u64 m = n + (e && e->stream.open ? e->stream.held : 0);
+  return b2_bound(m) + 1024ull * (m / 40000 + 16) + 16;
+}
+
+int b2_stream_begin(b2_encoder *e, int64_t size_hint, uint64_t window_bytes) {
+  if (!e) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  StreamState &S = e->stream;
+  if (S.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is already open on this handle");
+  const u64 W = window_bytes ? window_bytes : 512ull << 20;
+  if (W < (1ull << 20)) B2_FAIL(B2_ERR_ARGUMENT, "window_bytes below 1 MiB");
+  if (W > (1ull << 40)) B2_FAIL(B2_ERR_ARGUMENT, "window_bytes above 1 TiB");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  const u64 M = b2_shard_margin(e->level);
+  const u64 bytes = W + M + 256;
+  if (S.buf_bytes != bytes) {
+    for (int i = 0; i < 2; i++) { if (S.buf[i]) cudaFree(S.buf[i]); S.buf[i] = nullptr; }
+    S.buf_bytes = 0;
+    for (int i = 0; i < 2; i++) {
+      const cudaError_t ce = cudaMalloc((void **)&S.buf[i], bytes);
+      if (ce != cudaSuccess) {
+        for (int j = 0; j < 2; j++) { if (S.buf[j]) cudaFree(S.buf[j]); S.buf[j] = nullptr; }
+        B2_FAIL(B2_ERR_ALLOC, cudaGetErrorString(ce));
+      }
+    }
+    S.buf_bytes = bytes;
+  }
+  S.hint = size_hint; S.window = W; S.margin = M;
+  S.cur = 0; S.base = 0; S.held = 0; S.bit = 32; S.crc = 0; S.out_end = 0; S.tail = 0;
+  S.trace.clear();
+  e->stats.streams++;
+  S.open = true;
+  return 0;
+}
+
+int b2_stream_write(b2_encoder *e, const uint8_t *in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+  if (!e || !out_len || (n && !in) || !out) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  StreamState &S = e->stream;
+  if (!S.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_stream_write without b2_stream_begin");
+  *out_len = 0;
+  if (out_cap < b2_stream_bound(e, n)) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "output buffer below b2_stream_bound");
+  const u64 out0 = S.out_end;
+  auto run = [&]() -> int {
+    B2_CUDA_CHECK(cudaSetDevice(e->device));
+    const u64 full = S.window + S.margin;
+    u64 taken = 0;
+    for (;;) {
+      const u64 k = std::min<u64>(full - S.held, n - taken);
+      B2_TRY(stream_upload(e, S.cur, S.held, in + taken, k));
+      S.held += k; taken += k;
+      if (S.held < full) return 0;
+      B2_TRY(stream_window(e, false, in, n, &taken, out, out_cap, out0));
+    }
+  };
+  const int rc = run();
+  if (rc) { const std::string msg = g_last_error; stream_close(e); g_last_error = msg; return rc; }
+  B2_CUDA_CHECK(cudaStreamSynchronize(e->cst));          // the caller may reuse `in` once this returns
+  *out_len = S.out_end - out0;
+  return 0;
+}
+
+int b2_stream_end(b2_encoder *e, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+  if (!e || !out_len || !out) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  StreamState &S = e->stream;
+  if (!S.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_stream_end without b2_stream_begin");
+  *out_len = 0;
+  if (out_cap < b2_stream_bound(e, 0)) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "output buffer below b2_stream_bound");
+  const u64 out0 = S.out_end;
+  u64 taken = 0;
+  int rc = cudaSetDevice(e->device) == cudaSuccess ? 0 : B2_ERR_CUDA;
+  if (rc) b2_set_error(__FILE__, __LINE__, "cudaSetDevice");
+  if (!rc) rc = stream_window(e, true, nullptr, 0, &taken, out, out_cap, out0);
+  const std::string msg = g_last_error;
+  stream_close(e);
+  if (rc) { g_last_error = msg; return rc; }
+  e->trace.swap(S.trace);
+  S.trace.clear();
+  *out_len = S.out_end - out0;
+  return 0;
+}
+
+int b2_stream_abort(b2_encoder *e) {
+  if (!e) return B2_ERR_ARGUMENT;
+  if (e->stream.open) stream_close(e);
+  return 0;
+}
 
 // One stream over the devices of several handles of this process: the north star's block-wise sharding
 // (per-device streams, pinned host buffers, no collective).  One host thread per handle.
@@ -1308,6 +1545,7 @@ int b2_encode_stream_multi(b2_encoder **encs, int n_encs, const uint8_t *in, uin
                            uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
   if (!encs || n_encs < 1 || !out_len || (n && !in)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
   for (int i = 0; i < n_encs; i++) if (!encs[i] || encs[i]->level != encs[0]->level) B2_FAIL(B2_ERR_ARGUMENT, "handles must share the block size");
+  for (int i = 0; i < n_encs; i++) B2_NO_STREAM(encs[i]);
   const int level = encs[0]->level;
   u64 min_share = 64ull << 20;
   if (const char *sv = getenv("B2GPU_SHARD_MIN_BYTES")) { long long v = atoll(sv); if (v >= 65536) min_share = (u64)v; }
@@ -1384,6 +1622,7 @@ int b2_encode_stream_multi(b2_encoder **encs, int n_encs, const uint8_t *in, uin
 int b2_verify_stream(b2_encoder *e, const uint8_t *stream, int stream_is_device, uint64_t n, const uint8_t *expect,
                      int expect_is_device, uint64_t expect_n, b2_verify_result *res) {
   if (!e || !res || (n && !stream)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   memset(res, 0, sizeof *res);
   res->first_bad_block = -1; res->mismatch_at = ~0ull;
   B2_CUDA_CHECK(cudaSetDevice(e->device));
@@ -1522,6 +1761,7 @@ uint64_t b2_zip_bound(uint32_t n_entries, uint64_t total_name_bytes, uint64_t to
 
 int b2_zip_crc32(b2_encoder *e, const uint8_t *in, uint64_t n, uint32_t *crc) {
   if (!e || !crc || (n && !in)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   B2_TRY(e->d_in.ensure(n + 256));
   if (n) B2_CUDA_CHECK(cudaMemcpyAsync(e->d_in.p, in, n, cudaMemcpyHostToDevice, e->st));
@@ -1535,6 +1775,7 @@ int b2_zip_create(b2_encoder *e, uint32_t n_entries, const uint8_t *in, const ui
                   const char *names, const uint32_t *name_offsets, const uint32_t *dos_times, const uint32_t *flags,
                   int duplicates, uint8_t *out, uint64_t out_cap, uint64_t *out_len, b2_zip_entry_info *info) {
   if (!e || !out_len || (n_entries && (!in_offsets || !sizes || !names || !name_offsets))) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   // entry names: back slashes become forward slashes (Unixify, zip-create.adb:180-192)
   std::vector<std::string> nm(n_entries);
@@ -1704,6 +1945,7 @@ int b2_dbg_block(b2_encoder *e, const uint8_t *raw, uint32_t len, uint8_t *rle_o
                  uint16_t *mtf_out, uint8_t *sel_out, uint8_t *lens_out, uint8_t *bits_out, uint64_t bits_cap,
                  b2_block_info *info) {
   if (!e || (len && !raw)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  B2_NO_STREAM(e);
   B2_CUDA_CHECK(cudaSetDevice(e->device));
   Workspace *w = e->ws[0];
   cudaStream_t st = w->st;

@@ -76,4 +76,30 @@ void Encode(ReadByte Read_Byte, MoreBytes More_Bytes, WriteByte Write_Byte,
   for (uint64_t i = 0; i < out_len; i++) Write_Byte(out[i]);  // may throw (Compression_inefficient): the handle is back in the pool
 }
 
+// The same Encode, streaming: bytes are read into a 16 MiB staging buffer and handed to the device a buffer at a
+// time (b2_stream_write), and the bytes that are final go out through Write_Byte after every buffer, so memory does not
+// grow with the input.  Byte-identical to Encode.  An exception out of a callback aborts the handle's stream
+// (b2_stream_abort) before it propagates; the handle goes back to the pool.  window_bytes: see b2_stream_begin.
+template <class ReadByte, class MoreBytes, class WriteByte>
+void Encode_Streamed(ReadByte Read_Byte, MoreBytes More_Bytes, WriteByte Write_Byte,
+                     Compression_Option option = block_900k, Stream_Size_Type size_hint = unknown_size, int device = 0,
+                     uint64_t window_bytes = 0) {
+  b2_encoder *enc = Handle_Pool::instance().take((int)option, device);
+  struct Guard { int l, d; b2_encoder *e; ~Guard() { b2_stream_abort(e); Handle_Pool::instance().give(l, d, e); } } guard{(int)option, device, enc};
+  if (b2_stream_begin(enc, size_hint, window_bytes) != B2_OK) throw b2gpu_error(std::string("b2_stream_begin: ") + b2_last_error());
+  std::vector<uint8_t> in(16u << 20), out;
+  uint64_t out_len = 0;
+  for (bool more = true; more;) {
+    size_t n = 0;
+    while (n < in.size() && (more = More_Bytes())) in[n++] = Read_Byte();
+    out.resize(b2_stream_bound(enc, n));
+    if (b2_stream_write(enc, in.data(), n, out.data(), out.size(), &out_len) != B2_OK)
+      throw b2gpu_error(std::string("b2_stream_write: ") + b2_last_error());
+    for (uint64_t i = 0; i < out_len; i++) Write_Byte(out[i]);
+  }
+  out.resize(b2_stream_bound(enc, 0));
+  if (b2_stream_end(enc, out.data(), out.size(), &out_len) != B2_OK) throw b2gpu_error(std::string("b2_stream_end: ") + b2_last_error());
+  for (uint64_t i = 0; i < out_len; i++) Write_Byte(out[i]);
+}
+
 }  // namespace bzip2_encoding
