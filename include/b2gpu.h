@@ -300,6 +300,15 @@ B2_API int b2_get_trace(b2_encoder *enc, b2_chunk_trace *out, uint64_t cap, uint
 /* Segment_by_Entropy cut list of one chunk of the last call (profile 0 = segmented_1, 1 = segmented_2). */
 B2_API int b2_get_segments(b2_encoder *enc, uint64_t chunk, int profile, uint32_t *cuts, uint32_t cap, uint32_t *n);
 
+/* Segment_by_Entropy of one chunk of 0 < len <= 9 000 000 raw bytes by the device kernel, as one CTA: both cut lists
+ * (n0 / n1 cuts; the first min (n, cap) of them are written), the running entropy sum after every step
+ * (series[k] = the sum after step 16 001 + k of the reference, len - 16 000 values when the first profile is active,
+ * none when len <= 20 000; may be NULL) and the paths the replay took (may be NULL): batches of 256 steps that started
+ * on one binade, on two binades, failed predictions (restarts), batches finished by the literal chain of adds. */
+B2_API int b2_dbg_segment(b2_encoder *enc, const uint8_t *raw, uint64_t len, uint32_t *cuts0, uint32_t *n0,
+                          uint32_t *cuts1, uint32_t *n1, uint32_t cap, double *series, uint64_t series_cap,
+                          uint32_t *paths);
+
 #ifdef __cplusplus
 }
 #endif

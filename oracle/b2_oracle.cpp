@@ -275,9 +275,12 @@ void prepare_codes(const u32 *len, u32 *code, int n, int max_huffman_bits) {
 // data_segmentation.adb:39-105 — entropy change-point detector, FP64, libm log.
 // threshold is a Float (single precision) generic formal, widened (ads:43).
 // Returns ascending 1-based end indices; last = len (if len > 0).
+// series (optional): the running sum after the initial window (i = window_size) and after every
+// later step, at the point where it is tested against the threshold (tests/test_emu_segment.py).
 // ---------------------------------------------------------------------------
 void segment_by_entropy(const u8 *buffer /*0-based*/, i32 len, float discrepancy_threshold,
-                        i32 index_threshold, i32 window_size, std::vector<i32> &seg) {
+                        i32 index_threshold, i32 window_size, std::vector<i32> &seg,
+                        std::vector<double> *series = nullptr) {
   typedef double Real;                                                   // :41 digits 15
   const Real inv_window_size = 1.0 / (Real)window_size;                  // :44
   i32 freq[256]; Real elem[256];
@@ -299,6 +302,7 @@ void segment_by_entropy(const u8 *buffer /*0-based*/, i32 len, float discrepancy
           }
         }
         entropy_mark = entropy;
+        if (series) series->push_back((Real)entropy);
       } else if (i > window_size) {                                      // :73-98
         entropy = entropy - elem[bt];
         Real p = (Real)freq[bt] * inv_window_size;
@@ -314,6 +318,7 @@ void segment_by_entropy(const u8 *buffer /*0-based*/, i32 len, float discrepancy
         } else {
           elem[bt] = 0.0;
         }
+        if (series) series->push_back((Real)entropy);
         if (std::fabs(entropy - entropy_mark) > (Real)discrepancy_threshold) {
           i32 seg_point = i - window_size;
           if (seg_point - index_mark > index_threshold) {
@@ -1369,6 +1374,19 @@ int orc_segment(const u8 *raw, u32 len, int profile, u32 *cuts, u32 cap, u32 *n_
   *n_cuts = (u32)seg.size();
   for (size_t i = 0; i < seg.size() && i < cap; i++) cuts[i] = (u32)seg[i];
   return seg.size() > cap ? 2 : 0;
+}
+
+// The running entropy sum of Segment_by_Entropy (window 16_000; both profiles share it): *init after the
+// first window, series[k] after step k (reference i = 16_001 + k).  Empty when len <= 20_000: the loop
+// of the reference does not run (data_segmentation.adb:58).  Returns 2 when cap is too small.
+int orc_entropy_series(const u8 *raw, u32 len, double *init, double *series, u64 cap, u64 *n) {
+  std::vector<i32> seg;
+  std::vector<double> all;
+  segment_by_entropy(raw, (i32)len, 0.6f, 4000, 16000, seg, &all);
+  *init = all.empty() ? 0.0 : all[0];
+  *n = all.empty() ? 0 : all.size() - 1;
+  for (u64 k = 0; k < *n && k < cap; k++) series[k] = all[k + 1];
+  return *n > cap ? 2 : 0;
 }
 
 int orc_llhc(const u32 *freq, int n, int max_bits, u32 *lens) {

@@ -17,6 +17,7 @@
 #include <sched.h>
 
 #include <atomic>
+#include <cmath>
 #include <cstdint>
 #include <cstring>
 #include <functional>
@@ -27,6 +28,7 @@ struct EmuCta {
   pthread_barrier_t cta_bar;
   pthread_barrier_t warp_bar[32];
   uint32_t xchg[32][32];
+  int or_word = 0;                 // __syncthreads_or
   std::vector<unsigned char> smem;
 };
 static thread_local EmuCta *emu_cta = nullptr;
@@ -37,6 +39,18 @@ inline void emu_yield() { sched_yield(); }
 inline unsigned char *emu_dynamic_smem() { return emu_cta->smem.data(); }
 
 inline void __syncthreads() { pthread_barrier_wait(&emu_cta->cta_bar); }
+// every thread ORs its predicate into the CTA's word between two barriers; a third keeps the word until all have
+// read it, and thread 0 clears it before anyone can pass the first barrier of the next call
+inline int __syncthreads_or(int p) {
+  int *w = &emu_cta->or_word;
+  __syncthreads();
+  if (p) __atomic_fetch_or(w, 1, __ATOMIC_RELAXED);
+  __syncthreads();
+  const int r = __atomic_load_n(w, __ATOMIC_RELAXED);
+  __syncthreads();
+  if (threadIdx.x == 0) __atomic_store_n(w, 0, __ATOMIC_RELAXED);
+  return r;
+}
 inline void __syncwarp(unsigned = 0xffffffffu) { pthread_barrier_wait(&emu_cta->warp_bar[threadIdx.x >> 5]); }
 // every lane of the warp deposits a word, then reads all 32
 inline void emu_exchange(uint32_t v, uint32_t out[32]) {
@@ -66,8 +80,33 @@ inline uint32_t __shfl_up_sync(unsigned, uint32_t v, unsigned d) {
   const unsigned l = threadIdx.x & 31;
   return l >= d ? o[l - d] : v;
 }
+// 32-bit signed, 64-bit and double shuffles move every bit (two exchanges of the halves); any other argument type
+// would be converted to uint32_t and silently lose bits, so it does not compile
+inline int32_t __shfl_sync(unsigned m, int32_t v, unsigned src) { return (int32_t)__shfl_sync(m, (uint32_t)v, src); }
+inline int32_t __shfl_up_sync(unsigned m, int32_t v, unsigned d) { return (int32_t)__shfl_up_sync(m, (uint32_t)v, d); }
+inline uint64_t emu_shfl64(uint64_t v, unsigned src) { return (uint64_t)__shfl_sync(0xffffffffu, (uint32_t)v, src) | ((uint64_t)__shfl_sync(0xffffffffu, (uint32_t)(v >> 32), src) << 32); }
+inline uint64_t emu_shfl_up64(uint64_t v, unsigned d) { return (uint64_t)__shfl_up_sync(0xffffffffu, (uint32_t)v, d) | ((uint64_t)__shfl_up_sync(0xffffffffu, (uint32_t)(v >> 32), d) << 32); }
+inline long long __shfl_sync(unsigned, long long v, unsigned src) { return (long long)emu_shfl64((uint64_t)v, src); }
+inline long long __shfl_up_sync(unsigned, long long v, unsigned d) { return (long long)emu_shfl_up64((uint64_t)v, d); }
+inline unsigned long long __shfl_sync(unsigned, unsigned long long v, unsigned src) { return emu_shfl64(v, src); }
+inline unsigned long long __shfl_up_sync(unsigned, unsigned long long v, unsigned d) { return emu_shfl_up64(v, d); }
+inline double __shfl_sync(unsigned, double v, unsigned src) { uint64_t b; std::memcpy(&b, &v, 8); b = emu_shfl64(b, src); std::memcpy(&v, &b, 8); return v; }
+inline double __shfl_up_sync(unsigned, double v, unsigned d) { uint64_t b; std::memcpy(&b, &v, 8); b = emu_shfl_up64(b, d); std::memcpy(&v, &b, 8); return v; }
+template <class T> T __shfl_sync(unsigned, T, unsigned) = delete;
+template <class T> T __shfl_up_sync(unsigned, T, unsigned) = delete;
 inline uint32_t __shfl_xor_sync(unsigned, uint32_t v, unsigned x) { uint32_t o[32]; emu_exchange(v, o); return o[(threadIdx.x & 31) ^ x]; }
 inline int __popc(uint32_t x) { return __builtin_popcount(x); }
+// per byte: 0xFF where the bytes of a and b are equal
+inline uint32_t __vcmpeq4(uint32_t a, uint32_t b) {
+  uint32_t r = 0;
+  for (int k = 0; k < 32; k += 8) r |= (((a >> k) & 0xFFu) == ((b >> k) & 0xFFu) ? 0xFFu : 0u) << k;
+  return r;
+}
+// IEEE double adds, round to nearest even (the build uses -ffp-contract=off: nothing is fused)
+inline double __dadd_rn(double a, double b) { return a + b; }
+inline double __dsub_rn(double a, double b) { return a - b; }
+inline long long __double_as_longlong(double x) { long long r; std::memcpy(&r, &x, 8); return r; }
+inline double __longlong_as_double(long long x) { double r; std::memcpy(&r, &x, 8); return r; }
 inline int __ffs(uint32_t x) { return __builtin_ffs((int)x); }
 inline int __clz(uint32_t x) { return x ? __builtin_clz(x) : 32; }
 
@@ -114,5 +153,16 @@ inline void emu_launch(unsigned grid, unsigned block, size_t smem_bytes, unsigne
 inline bool __any_sync(unsigned, bool p) { return __ballot_sync(0xffffffffu, p) != 0u; }
 inline uint32_t atomicOr(uint32_t *p, uint32_t v) { return __atomic_fetch_or(p, v, __ATOMIC_RELAXED); }
 inline uint32_t atomicAdd(uint32_t *p, uint32_t v) { return __atomic_fetch_add(p, v, __ATOMIC_RELAXED); }
+inline uint32_t atomicMin(uint32_t *p, uint32_t v) {
+  uint32_t old = __atomic_load_n(p, __ATOMIC_RELAXED);
+  while (v < old && !__atomic_compare_exchange_n(p, &old, v, true, __ATOMIC_RELAXED, __ATOMIC_RELAXED)) {}
+  return old;
+}
+// loads past the L1 / fences / back-off: no reordering or caching to model for one CTA
+template <class T> inline T __ldcg(const T *p) { return *p; }
+inline void __threadfence() { std::atomic_thread_fence(std::memory_order_seq_cst); }
+inline void __nanosleep(unsigned) { emu_yield(); }
+using std::fabs;
+using std::floor;
 using std::max;
 using std::min;

@@ -110,6 +110,20 @@ def segment(data, profile):
     return cuts[:n.value].copy()
 
 
+def entropy_series(data):
+    """Segment_by_Entropy's running FP64 sum: (sum after the first 16 000 bytes, float64 array of the sum after every
+    later step).  The series is empty when len(data) <= 20 000 (the reference's loop does not run)."""
+    a = _u8(data)
+    cap = max(a.size - 16_000, 1)
+    series = np.zeros(cap, np.float64)
+    init = C.c_double(0.0)
+    n = C.c_uint64(0)
+    rc = lib().orc_entropy_series(a.ctypes.data_as(C.c_void_p), C.c_uint32(a.size), C.byref(init),
+                                  series.ctypes.data_as(C.c_void_p), C.c_uint64(cap), C.byref(n))
+    assert rc == 0, rc
+    return init.value, series[:n.value].copy()
+
+
 def llhc(freq, max_bits):
     f = np.ascontiguousarray(freq, dtype=np.uint32)
     lens = np.zeros(f.size, np.uint32)

@@ -4,6 +4,7 @@ for the unique-result steps, by optimality checks, and by regression vectors und
 import bz2
 import hashlib
 import json
+import math
 import os
 import subprocess
 
@@ -198,6 +199,47 @@ def test_segmentation_detects_regime_changes():
     assert c1[-1] == d.size and c2[-1] == d.size and len(c1) > 1 and len(c2) > 1
     assert all(b - a > 4000 for a, b in zip(c1[:-2], c1[1:-1])) and all(b - a > 8000 for a, b in zip(c2[:-2], c2[1:-1]))
     assert len(orc.segment(d[:20_000], 0)) == 1          # len <= window + index_threshold: trivial (data_segmentation.adb:58)
+
+
+def test_entropy_series_is_the_segmentation_sum():
+    """orc.entropy_series records the sum of the very run that places the cuts: a literal Python chain of the four
+    IEEE adds per step (the reference's order, data_segmentation.adb:63-90) gives it bit for bit, and the threshold
+    rule of :91-97 applied to it gives both cut lists."""
+    d = np.concatenate([datagen.text(40_000, 21), datagen.random_bytes(30_000, 22), np.zeros(30_000, np.uint8)])
+    init, series = orc.entropy_series(d)
+    assert series.size == d.size - 16_000
+    inv = 1.0 / 16000.0                                     # p = freq * inv_window_size (:44, :49)
+    T = [0.0] + [-((c * inv) * math.log(c * inv)) for c in range(1, 16002)]
+    f = [0] * 256
+    for b in d[:16_000]:
+        f[b] += 1
+    e = 0.0
+    for b in range(256):
+        if f[b]:
+            e = e + T[f[b]]
+    assert e == init
+    mine = np.zeros(series.size)
+    for k in range(series.size):
+        bn, bo = int(d[16_000 + k]), int(d[k])
+        e = e - T[f[bn]]
+        f[bn] += 1
+        e = e + T[f[bn]]
+        e = e - T[f[bo]]
+        f[bo] -= 1
+        e = e + T[f[bo]]
+        mine[k] = e
+    assert np.array_equal(mine.view(np.uint64), series.view(np.uint64))
+    for profile, thr, ith in ((0, 0.6, 4000), (1, 0.4, 8000)):
+        thr = float(np.float32(thr))
+        cuts, mark, imark = [], init, 1
+        if d.size > 16_000 + ith:
+            for k, v in enumerate(series):
+                sp = k + 1
+                if abs(v - mark) > thr and sp - imark > ith:
+                    cuts.append(sp)
+                    imark, mark = sp, v
+        assert cuts + [d.size] == list(orc.segment(d, profile)), profile
+    assert orc.entropy_series(d[:20_000])[1].size == 0 and orc.entropy_series(d[:20_001])[1].size == 4_001
 
 
 def test_crc_is_bzip2_crc():

@@ -63,7 +63,7 @@ EXPORTS = ["b2_create", "b2_destroy", "b2_bound", "b2_encode_stream", "b2_encode
            "b2_zip_bound", "b2_zip_create", "b2_zip_crc32",
            "b2_shard_margin", "b2_shard_plan", "b2_shard_open", "b2_shard_cut", "b2_shard_encode", "b2_shard_resolve",
            "b2_shard_finish", "b2_encode_stream_multi", "b2_set_progress", "b2_verify_stream",
-           "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort"]
+           "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort", "b2_dbg_segment"]
 
 _lib = None
 
@@ -99,6 +99,8 @@ def lib():
         _lib.b2_dbg_block.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 6 + [C.c_uint64, C.POINTER(BlockInfo)]
         _lib.b2_get_trace.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         _lib.b2_get_segments.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
+        _lib.b2_dbg_segment.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p,
+                                        C.POINTER(C.c_uint32), C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]
         _lib.b2_set_progress.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         _lib.b2_verify_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_int, C.c_uint64, C.POINTER(VerifyResult)]
         _lib.b2_shard_margin.restype = C.c_uint64
@@ -342,6 +344,20 @@ class Encoder:
         n = C.c_uint32(0)
         _check(lib().b2_get_segments(self._h, chunk, profile, cuts.ctypes.data, cuts.size, C.byref(n)))
         return cuts[:n.value].copy()
+
+    def dbg_segment(self, data):
+        """Segment_by_Entropy of one chunk by the device kernel: dict(cuts=[profile 0, profile 1] as uint32 arrays,
+        series=float64 sum after every step (empty when len <= 20 000), paths=uint32[4]: batches started on one
+        binade, on two binades, restarts, batches finished by the literal chain)."""
+        a = _u8(data)
+        cuts = np.zeros((2, 2304), np.uint32)
+        n0, n1 = C.c_uint32(0), C.c_uint32(0)
+        series = np.zeros(max(a.size - 16_000, 1), np.float64)
+        paths = np.zeros(4, np.uint32)
+        _check(lib().b2_dbg_segment(self._h, a.ctypes.data, a.size, cuts[0].ctypes.data, C.byref(n0), cuts[1].ctypes.data,
+                                    C.byref(n1), cuts.shape[1], series.ctypes.data, series.size, paths.ctypes.data))
+        steps = a.size - 16_000 if a.size > 20_000 else 0
+        return dict(cuts=[cuts[0, :n0.value].copy(), cuts[1, :n1.value].copy()], series=series[:steps].copy(), paths=paths)
 
     def dbg_block(self, data):
         a = _u8(data)

@@ -547,7 +547,7 @@ int encode_streams(b2_encoder *e, const u8 *d_in, std::vector<StreamDesc> &strea
         e->launches_other += 5;
         if (follow) {
           B2_CUDA_CHECK(cudaStreamWaitEvent(e->st2, e->ev_fork, 0));
-          B2_TRY(b2k_segment(e->st2, d_in + S.off, e->d_chunks.p, max_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, e->d_scalars.p + 12));
+          B2_TRY(b2k_segment(e->st2, d_in + S.off, e->d_chunks.p, max_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, e->d_scalars.p + 12, nullptr, nullptr));
           B2_CUDA_CHECK(cudaEventRecord(e->ev_join, e->st2));
           e->launches_other += 1;
           followed = true;
@@ -593,7 +593,7 @@ int encode_chunks(b2_encoder *e, const u8 *d_in, std::vector<StreamDesc> &stream
       if (!followed) {
         B2_TRY(e->d_seg.ensure((size_t)n_chunks * 2 * B2_MAX_SEG));
         B2_TRY(e->d_nseg.ensure((size_t)n_chunks * 2));
-        B2_TRY(b2k_segment(st, d_in, e->d_chunks.p, n_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, nullptr));
+        B2_TRY(b2k_segment(st, d_in, e->d_chunks.p, n_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, nullptr, nullptr, nullptr));
         e->launches_other += 1;
       }
     }
@@ -620,7 +620,7 @@ int encode_chunks(b2_encoder *e, const u8 *d_in, std::vector<StreamDesc> &stream
         // segment every chunk again now that the chain is complete
         B2_CUDA_CHECK(cudaStreamSynchronize(e->st2));
         B2_CUDA_CHECK(cudaMemcpyAsync(e->d_chunks.p, e->chunks.data(), n_chunks * sizeof(B2Chunk), cudaMemcpyHostToDevice, st));
-        B2_TRY(b2k_segment(st, d_in, e->d_chunks.p, n_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, nullptr));
+        B2_TRY(b2k_segment(st, d_in, e->d_chunks.p, n_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, nullptr, nullptr, nullptr));
         e->launches_other += 1;
         followed = false;
         continue;
@@ -1199,7 +1199,7 @@ int shard_cut(b2_encoder *e, u64 entry, u64 *handoff) {
   e->launches_other += 1;
   if (follow) {
     B2_CUDA_CHECK(cudaStreamWaitEvent(e->st2, e->ev_fork, 0));
-    B2_TRY(b2k_segment(e->st2, sh.d_in, e->d_chunks.p, max_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, e->d_scalars.p + 12));
+    B2_TRY(b2k_segment(e->st2, sh.d_in, e->d_chunks.p, max_chunks, e->d_T.p, e->d_seg.p, e->d_nseg.p, e->d_scalars.p + 12, nullptr, nullptr));
     B2_CUDA_CHECK(cudaEventRecord(e->ev_join, e->st2));
     e->launches_other += 1;
   }
@@ -1980,6 +1980,45 @@ int b2_dbg_block(b2_encoder *e, const uint8_t *raw, uint32_t len, uint8_t *rle_o
     info->n_used = b.n_used; info->n_sel = b.n_groups; info->ec_count = (u32)ec; info->max_len = (u32)max_len;
     info->sample_width = (u32)sw; info->cost = b.best_cost; info->pad = 0; info->bits = b.nbits;
   }
+  return 0;
+}
+
+int b2_dbg_segment(b2_encoder *e, const uint8_t *raw, uint64_t len, uint32_t *cuts0, uint32_t *n0, uint32_t *cuts1,
+                   uint32_t *n1, uint32_t cap, double *series, uint64_t series_cap, uint32_t *paths) {
+  if (!e || !raw || len == 0 || len > 9000000 || !n0 || !n1 || (cap && (!cuts0 || !cuts1))) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  const u64 steps = len > 20000 ? len - 16000 : 0;      // window 16 000; no step below window + 4 000 (b2_segment.cuh)
+  if (series && series_cap < steps) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "series too small");
+  B2_NO_STREAM(e);
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  cudaStream_t st = e->st;
+  struct Taps { DevBuf<double> series; DevBuf<u32> paths; ~Taps() { series.release(); paths.release(); } } taps;
+  B2_TRY(e->d_in.ensure((size_t)len + 256));
+  B2_CUDA_CHECK(cudaMemcpyAsync(e->d_in.p, raw, len, cudaMemcpyHostToDevice, st));
+  B2_CUDA_CHECK(cudaMemsetAsync(e->d_in.p + len, 0, 128, st));
+  const B2Chunk chunk{0, (u32)len, 0, 0, 0};
+  B2_TRY(e->d_chunks.ensure(1));
+  B2_CUDA_CHECK(cudaMemcpyAsync(e->d_chunks.p, &chunk, sizeof chunk, cudaMemcpyHostToDevice, st));
+  B2_TRY(e->d_seg.ensure(2 * B2_MAX_SEG));
+  B2_TRY(e->d_nseg.ensure(2));
+  if (series && steps) B2_TRY(taps.series.ensure(steps));
+  if (paths) {
+    B2_TRY(taps.paths.ensure(4));
+    B2_CUDA_CHECK(cudaMemsetAsync(taps.paths.p, 0, 4 * sizeof(u32), st));
+  }
+  B2_TRY(b2k_segment(st, e->d_in.p, e->d_chunks.p, 1, e->d_T.p, e->d_seg.p, e->d_nseg.p, nullptr,
+                     series && steps ? taps.series.p : nullptr, paths ? taps.paths.p : nullptr));
+  u32 ns[2] = {0, 0};
+  B2_CUDA_CHECK(cudaMemcpyAsync(ns, e->d_nseg.p, sizeof ns, cudaMemcpyDeviceToHost, st));
+  if (series && steps) B2_CUDA_CHECK(cudaMemcpyAsync(series, taps.series.p, steps * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (paths) B2_CUDA_CHECK(cudaMemcpyAsync(paths, taps.paths.p, 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+  B2_CUDA_CHECK(cudaStreamSynchronize(st));
+  uint32_t *cuts[2] = {cuts0, cuts1};
+  for (int p = 0; p < 2; p++) {
+    if (ns[p] > B2_MAX_SEG) B2_FAIL(B2_ERR_INTERNAL, "segment table overflow");
+    const u32 k = std::min(ns[p], cap);
+    if (k) B2_CUDA_CHECK(cudaMemcpy(cuts[p], e->d_seg.p + (size_t)p * B2_MAX_SEG, k * sizeof(u32), cudaMemcpyDeviceToHost));
+  }
+  *n0 = ns[0]; *n1 = ns[1];
   return 0;
 }
 

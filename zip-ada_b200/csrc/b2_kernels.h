@@ -40,7 +40,7 @@ int b2k_cut_chain(cudaStream_t st, const u8 *d_in, u64 n, i64 size_hint, int lev
 #define B2_SEG_GAVE_UP 0xFFFFFFFDu     // a CTA following the chunk chain never saw its chunk (time-sliced GPU): segment again afterwards
 #define B2_SEG_PENDING 0xFEFEFEFEu
 int b2k_segment(cudaStream_t st, const u8 *d_in, const B2Chunk *d_chunks, u32 n_chunks, const double *d_T,
-                u32 *d_seg, u32 *d_nseg, const u32 *d_progress);
+                u32 *d_seg, u32 *d_nseg, const u32 *d_progress, double *d_dbg_series, u32 *d_dbg_paths);   // taps: b2_segment.cuh
 // b2_rle1.cu
 void b2k_make_crc_tables(B2CrcTables *t);
 int b2k_rle1(cudaStream_t st, const u8 *d_in, B2Job *d_jobs, u32 n_jobs, u8 *d_text, const B2CrcTables *d_ct);
