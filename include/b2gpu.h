@@ -143,7 +143,7 @@ B2_API int b2_encode_stream_multi(b2_encoder **encs, int n_encs, const uint8_t *
  * The concatenation of every out of b2_stream_write and b2_stream_end is byte-identical to what
  * b2_encode_stream gives for the concatenated input and the same size_hint.
  *   - One open stream per handle.  While it is open, every other call that uses the handle's device buffers
- *     (encode, batch, zip, shard, verify, zip_crc32, dbg) returns B2_ERR_ARGUMENT; b2_stream_*, b2_set_*,
+ *     (encode, batch, zip, shard, verify, zip_crc32, dbg, b2_zip_begin) returns B2_ERR_ARGUMENT; b2_stream_*, b2_set_*,
  *     b2_get_*, b2_reset_stats and b2_destroy are allowed.
  *   - The handle holds the bytes not yet encoded on the device, from the start of the next chunk.  When
  *     window_bytes + b2_shard_margin (level) of them are held, it encodes the chunks that start in the first
@@ -206,6 +206,54 @@ B2_API int b2_zip_create(b2_encoder *enc, uint32_t n_entries, const uint8_t *in,
                   const uint64_t *sizes, const char *names, const uint32_t *name_offsets,
                   const uint32_t *dos_times, const uint32_t *flags, int duplicates,
                   uint8_t *out, uint64_t out_cap, uint64_t *out_len, b2_zip_entry_info *info);
+
+/* ---- Archive side, one entry at a time (Zip.Create: Create_Archive, Add_Stream per entry, Finish) ----------------
+ * b2_zip_begin opens an archive on the handle; each b2_zip_add gives one whole entry; b2_zip_finish writes what is left
+ * and the central directory and closes it.
+ *   - Parity: the concatenation of every `out` of b2_zip_add and b2_zip_finish is byte-identical to what b2_zip_create
+ *     writes for the same entries, names, times, flags and duplicates, and `info` is the same, for every window_bytes
+ *     and every sequence of entry sizes.
+ *   - `in` holds the whole entry in host memory (it may be an mmap of a file); the caller may reuse it once the call
+ *     returns.
+ *   - An entry of at most W = window_bytes bytes (0 = 512 MiB; below 1 MiB is B2_ERR_ARGUMENT) is uploaded to a device
+ *     staging buffer and queued.  When the next entry would not fit (the queue would hold more than W bytes, or more
+ *     than max (32, W / 32 KiB) entries, or their 16-byte aligned placement would pass W + b2_shard_margin (level)),
+ *     the queue is encoded as one batch, as b2_zip_create encodes its entries, and its archive bytes (local headers
+ *     and payloads) go to `out`.
+ *   - An entry above W first writes the queue.  It is then one stream through the windows of b2_stream_* with
+ *     size_hint = its size, written behind its local header (whose length is known before compression and whose fields
+ *     are filled in at the end).  Its Zip CRC-32 is folded window by window; the Store fallback copies from `in`.
+ *   - `out` receives every entry the call finished: none, one or many.  out_cap below b2_zip_add_bound (enc, n,
+ *     name_bytes) (the queue plus the new entry) or b2_zip_finish_bound (enc) (the queue plus the central directory and
+ *     end records) returns B2_ERR_OUTPUT_TOO_SMALL before anything is taken; the call can be repeated.
+ *   - With B2_ZIP_ERROR_ON_DUPLICATE a name seen before returns B2_ERR_DUPLICATE_NAME; the entry is not added and the
+ *     archive stays open and unchanged.  Offsets in `info` are archive offsets; the Zip64 state (Check_Size) is carried
+ *     from call to call.
+ *   - Device memory is bounded by W, not by the archive: the input buffers are the two window buffers of b2_stream_*,
+ *     2 x (W + M + 256) bytes with M = b2_shard_margin (level), the queue staging in the first one.  A batch holds at
+ *     most W input bytes (the encode workspace, about 150 bytes per byte, DESIGN.md §3, §6b) and at most one entry per
+ *     32 KiB of W (each costs at most about 2 MB at level 9, whatever its size: 64 bytes per byte of W).  With the
+ *     fixed tables and the workspace floor of a small batch, the handle holds at most
+ *     2 x (W + M + 256) + 224 x W + 512 MiB bytes of device memory (DESIGN.md §7c).  Host memory holds the entry names
+ *     and the central directory, not the entries.
+ *   - One open archive per handle.  While it is open, the calls refused during a stream (b2_stream_begin included) return
+ *     B2_ERR_ARGUMENT; an archive is refused while a stream is open.
+ *   - b2_set_progress fires after every device batch with the archive's uncompressed bytes done and the bytes added so
+ *     far.  A bad argument is refused and changes nothing; any other error except B2_ERR_OUTPUT_TOO_SMALL and
+ *     B2_ERR_DUPLICATE_NAME, B2_ERR_ABORTED included, closes the archive; the handle stays usable.  An archive that
+ *     passes Zip's capacity (Zip_Capacity_Exceeded, Check_Size) returns B2_ERR_ARGUMENT, as b2_zip_create does, and
+ *     closes the archive. */
+B2_API int b2_zip_begin(b2_encoder *enc, int duplicates, uint64_t window_bytes);
+B2_API uint64_t b2_zip_add_bound(b2_encoder *enc, uint64_t n, uint32_t name_bytes);
+/* name: name_bytes bytes, '\\' becomes '/'; dos_time: Zip_Streams.Time; flags: B2_ZIP_* bits. */
+B2_API int b2_zip_add(b2_encoder *enc, const char *name, uint32_t name_bytes, uint32_t dos_time, uint32_t flags,
+                      const uint8_t *in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+B2_API uint64_t b2_zip_finish_bound(b2_encoder *enc);
+/* info (may be NULL when info_cap = 0) receives the first info_cap entries; n_entries (may be NULL) their number. */
+B2_API int b2_zip_finish(b2_encoder *enc, uint8_t *out, uint64_t out_cap, uint64_t *out_len,
+                         b2_zip_entry_info *info, uint64_t info_cap, uint64_t *n_entries);
+/* Closes the open archive, if any, discarding what it holds. */
+B2_API int b2_zip_abort(b2_encoder *enc);
 
 /* Zip CRC-32 of a host buffer, computed on the device (zip-crc_crypto.adb:31-61: Init, Update, Final). */
 B2_API int b2_zip_crc32(b2_encoder *enc, const uint8_t *in, uint64_t n, uint32_t *crc);

@@ -63,7 +63,8 @@ EXPORTS = ["b2_create", "b2_destroy", "b2_bound", "b2_encode_stream", "b2_encode
            "b2_zip_bound", "b2_zip_create", "b2_zip_crc32",
            "b2_shard_margin", "b2_shard_plan", "b2_shard_open", "b2_shard_cut", "b2_shard_encode", "b2_shard_resolve",
            "b2_shard_finish", "b2_encode_stream_multi", "b2_set_progress", "b2_verify_stream",
-           "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort", "b2_dbg_segment"]
+           "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort", "b2_dbg_segment",
+           "b2_zip_begin", "b2_zip_add_bound", "b2_zip_add", "b2_zip_finish_bound", "b2_zip_finish", "b2_zip_abort"]
 
 _lib = None
 
@@ -92,6 +93,16 @@ def lib():
         _lib.b2_zip_create.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64),
                                        C.c_void_p]
+        _lib.b2_zip_begin.argtypes = [C.c_void_p, C.c_int, C.c_uint64]
+        _lib.b2_zip_add_bound.restype = C.c_uint64
+        _lib.b2_zip_add_bound.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32]
+        _lib.b2_zip_add.argtypes = [C.c_void_p, C.c_char_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p,
+                                    C.c_uint64, C.POINTER(C.c_uint64)]
+        _lib.b2_zip_finish_bound.restype = C.c_uint64
+        _lib.b2_zip_finish_bound.argtypes = [C.c_void_p]
+        _lib.b2_zip_finish.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_void_p, C.c_uint64,
+                                       C.POINTER(C.c_uint64)]
+        _lib.b2_zip_abort.argtypes = [C.c_void_p]
         _lib.b2_zip_crc32.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint32)]
         _lib.b2_set_timing.argtypes = [C.c_void_p, C.c_int]
         _lib.b2_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
@@ -250,6 +261,14 @@ class Encoder:
         res = out[:out_len.value]
         return (res, [info[i] for i in range(n)]) if want_info else res
 
+    def zip_writer(self, duplicates=0, window=0):
+        """Opens an archive on the handle, written entry by entry (b2_zip_begin): `ZipWriter.add` and `ZipWriter.finish`
+        return the archive bytes finished so far; together they are `zip_create` of the same entries.  window: entries
+        of at most this many bytes are queued and encoded together, larger ones go through windows of this size
+        (0 = 512 MiB)."""
+        _check(lib().b2_zip_begin(self._h, int(duplicates), int(window)))
+        return ZipWriter(self)
+
     def zip_crc32(self, data):
         """Zip CRC-32 (zip-crc_crypto.adb:31-61) computed on the device."""
         a = _u8(data)
@@ -404,6 +423,58 @@ class Stream:
 
     def abort(self):
         _check(lib().b2_stream_abort(self.enc._h))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, *a):
+        if exc_type is not None:
+            self.abort()
+
+
+class ZipWriter:
+    """The open archive of an Encoder (Encoder.zip_writer).  After `finish`, `.info` holds the ZipEntryInfo of every
+    entry.  As a context manager it aborts the archive when the block raises, so that the handle can encode again."""
+
+    def __init__(self, enc):
+        self.enc = enc
+        self.info = None
+        self._n = 0                                                      # entries added
+        self._out = np.empty(0, dtype=np.uint8)                          # output buffer, reused from call to call
+
+    def _buffer(self, cap):
+        if self._out.size < cap:
+            self._out = np.empty(cap, dtype=np.uint8)
+        return self._out
+
+    def add(self, name, data, dos_time=None, unicode=False, read_only=False):
+        """Create.Add_Stream of one whole entry; returns the archive bytes this call finished (often none)."""
+        a = _u8(data)
+        nb = name.encode("utf-8") if isinstance(name, str) else bytes(name)
+        h = self.enc._h
+        cap = int(lib().b2_zip_add_bound(h, a.size, len(nb)))
+        out = self._buffer(cap)
+        out_len = C.c_uint64(0)
+        t = 16789 * 65536 if dos_time is None else int(dos_time)         # Zip_Streams.default_time
+        fl = (1 if unicode else 0) | (2 if read_only else 0)             # B2_ZIP_UNICODE_NAME, B2_ZIP_READ_ONLY
+        _check(lib().b2_zip_add(h, C.c_char_p(nb), len(nb), t, fl, a.ctypes.data if a.size else None, a.size, out.ctypes.data,
+                                out.size, C.byref(out_len)))
+        self._n += 1
+        return out[:out_len.value].tobytes()
+
+    def finish(self):
+        h = self.enc._h
+        cap = int(lib().b2_zip_finish_bound(h))
+        out = self._buffer(cap)
+        out_len, n = C.c_uint64(0), C.c_uint64(0)
+        info = (ZipEntryInfo * max(self._n, 1))()
+        _check(lib().b2_zip_finish(h, out.ctypes.data, out.size, C.byref(out_len), info, self._n, C.byref(n)))
+        self._out = np.empty(0, dtype=np.uint8)
+        self.info = [info[i] for i in range(n.value)]
+        return out[:out_len.value].tobytes()
+
+    def abort(self):
+        _check(lib().b2_zip_abort(self.enc._h))
 
     def __enter__(self):
         return self

@@ -15,6 +15,7 @@
 // b2_zip_create adds the archive side around the same machinery (Zip CRC-32, headers, Store fallback).
 #include "b2_common.cuh"
 #include "b2_kernels.h"
+#include "b2_zip_layout.h"
 #include "../../include/b2gpu.h"
 
 #include <algorithm>
@@ -40,8 +41,9 @@ void b2_set_error(const char *file, int line, const char *msg) {
 }
 #define B2_FAIL(code, msg) do { b2_set_error(__FILE__, __LINE__, msg); return code; } while (0)
 #define B2_TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
-// calls that use the handle's device buffers are refused while b2_stream_* owns them
-#define B2_NO_STREAM(e) do { if ((e)->stream.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is open on this handle (b2_stream_begin)"); } while (0)
+// calls that use the handle's device buffers are refused while b2_stream_* or b2_zip_begin .. finish own them
+#define B2_NO_STREAM(e) do { if ((e)->stream.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is open on this handle (b2_stream_begin)"); \
+                             if ((e)->zip.open) B2_FAIL(B2_ERR_ARGUMENT, "an archive is open on this handle (b2_zip_begin)"); } while (0)
 
 namespace {
 
@@ -160,10 +162,26 @@ struct StreamState {
   std::vector<b2_chunk_trace> trace;   // every chunk of the stream so far, stream offsets
 };
 
+// One archive written entry by entry (b2_zip_*, DESIGN.md §7c).  Small entries are queued in stream.buf[0]; an entry
+// above the window goes through the windows of b2_stream_* (the StreamState) with its own size as size_hint.
+struct ZipQueued { std::string name; u64 off, n; u32 time, flags; };
+struct ZipState {
+  bool open = false;
+  int duplicates = 0;
+  b2zip::ZipLayout layout;               // pos = archive bytes written to an `out` so far
+  std::unordered_set<std::string> names; // with B2_ZIP_ERROR_ON_DUPLICATE
+  std::vector<ZipQueued> queue;          // entries uploaded, not encoded yet
+  u64 q_end = 0, q_bytes = 0;            // staging bytes in use (16-byte aligned placement), input bytes queued
+  u64 q_bound = 0;                       // archive bytes the queue can become
+  u64 cd_bound = 0;                      // central directory bytes, at most, of every entry added
+  u64 done = 0, added = 0;               // uncompressed bytes encoded, added
+};
+
 struct b2_encoder {
   int level = 9, device = 0;
   ShardState shard;
   StreamState stream;
+  ZipState zip;
   cudaStream_t cst = nullptr;           // uploads of b2_stream_write, overlapping the encode of the window before
   cudaEvent_t ev_up = nullptr;          // recorded on cst after every upload
   b2_progress_fn progress = nullptr;    // called on the calling thread between batches; non-zero return aborts
@@ -932,14 +950,6 @@ int zip_crc_device(b2_encoder *e, const u8 *d_in, u32 n_entries, const u64 *offs
   return 0;
 }
 
-struct ByteSink {                                   // little-endian fields (zip-headers.adb:54-70)
-  std::vector<u8> b;
-  void u16le(u32 v) { b.push_back((u8)v); b.push_back((u8)(v >> 8)); }
-  void u32le(u64 v) { for (int k = 0; k < 4; k++) b.push_back((u8)(v >> (8 * k))); }
-  void u64le(u64 v) { for (int k = 0; k < 8; k++) b.push_back((u8)(v >> (8 * k))); }
-  void sig(u8 c1, u8 c2) { b.push_back(0x50); b.push_back(0x4B); b.push_back(c1); b.push_back(c2); }
-  void str(const std::string &s) { b.insert(b.end(), s.begin(), s.end()); }
-};
 struct HeaderSpan { u64 dst; std::vector<u8> bytes; };
 }  // namespace
 
@@ -1448,23 +1458,12 @@ int stream_window(b2_encoder *e, bool last, const u8 *in, u64 n, u64 *taken, u8 
   S.cur = nxt; S.base = handoff; S.held = next_held;
   return 0;
 }
-}  // namespace
-
-extern "C" {
-
-uint64_t b2_stream_bound(b2_encoder *e, uint64_t n) {
-  const u64 m = n + (e && e->stream.open ? e->stream.held : 0);
-  return b2_bound(m) + 1024ull * (m / 40000 + 16) + 16;
-}
-
-int b2_stream_begin(b2_encoder *e, int64_t size_hint, uint64_t window_bytes) {
-  if (!e) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+// The two window buffers of W + M + 256 bytes (kept across streams and archives of the same W).
+int stream_buffers(b2_encoder *e, u64 window_bytes) {
   StreamState &S = e->stream;
-  if (S.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is already open on this handle");
   const u64 W = window_bytes ? window_bytes : 512ull << 20;
   if (W < (1ull << 20)) B2_FAIL(B2_ERR_ARGUMENT, "window_bytes below 1 MiB");
   if (W > (1ull << 40)) B2_FAIL(B2_ERR_ARGUMENT, "window_bytes above 1 TiB");
-  B2_CUDA_CHECK(cudaSetDevice(e->device));
   const u64 M = b2_shard_margin(e->level);
   const u64 bytes = W + M + 256;
   if (S.buf_bytes != bytes) {
@@ -1479,9 +1478,34 @@ int b2_stream_begin(b2_encoder *e, int64_t size_hint, uint64_t window_bytes) {
     }
     S.buf_bytes = bytes;
   }
-  S.hint = size_hint; S.window = W; S.margin = M;
+  S.window = W; S.margin = M;
+  return 0;
+}
+
+// A new stream of the window size of the buffers: nothing held, the first block behind "BZh<level>".
+void stream_reset(b2_encoder *e, i64 size_hint) {
+  StreamState &S = e->stream;
+  S.hint = size_hint;
   S.cur = 0; S.base = 0; S.held = 0; S.bit = 32; S.crc = 0; S.out_end = 0; S.tail = 0;
   S.trace.clear();
+}
+}  // namespace
+
+extern "C" {
+
+uint64_t b2_stream_bound(b2_encoder *e, uint64_t n) {
+  const u64 m = n + (e && e->stream.open ? e->stream.held : 0);
+  return b2_bound(m) + 1024ull * (m / 40000 + 16) + 16;
+}
+
+int b2_stream_begin(b2_encoder *e, int64_t size_hint, uint64_t window_bytes) {
+  if (!e) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  StreamState &S = e->stream;
+  if (S.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is already open on this handle");
+  if (e->zip.open) B2_FAIL(B2_ERR_ARGUMENT, "an archive is open on this handle (b2_zip_begin)");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  B2_TRY(stream_buffers(e, window_bytes));
+  stream_reset(e, size_hint);
   e->stats.streams++;
   S.open = true;
   return 0;
@@ -1783,8 +1807,7 @@ int b2_zip_create(b2_encoder *e, uint32_t n_entries, const uint8_t *in, const ui
     std::unordered_set<std::string> seen;
     for (u32 i = 0; i < n_entries; i++) {
       if (name_offsets[i + 1] < name_offsets[i] || name_offsets[i + 1] - name_offsets[i] > 65535u) B2_FAIL(B2_ERR_ARGUMENT, "bad entry name length");
-      nm[i].assign(names + name_offsets[i], names + name_offsets[i + 1]);
-      for (char &c : nm[i]) if (c == '\\') c = '/';
+      nm[i] = b2zip::unixify(names + name_offsets[i], name_offsets[i + 1] - name_offsets[i]);
       if (duplicates == B2_ZIP_ERROR_ON_DUPLICATE && !seen.insert(nm[i]).second) {   // Duplicate_name (zip-create.adb:138-147)
         g_last_error = "Duplicate_name: Entry name = " + nm[i];
         return B2_ERR_DUPLICATE_NAME;
@@ -1808,85 +1831,30 @@ int b2_zip_create(b2_encoder *e, uint32_t n_entries, const uint8_t *in, const ui
   B2_CUDA_CHECK(cudaStreamSynchronize(e->st));
 
   // ---- layout: what Add_Stream (zip-create.adb:194-297) and Finish (:645-756) leave in the stream ----
-  const u64 four_gib = 1ull << 32, max_size = 0x1FFFFFFFFFFFFFFFull;
-  const u64 margin = 22 + 56 + 20 + 65536 + 10;                    // Check_Size (:161-179)
-  bool zip64 = false;
-  auto check_size = [&](u64 value) -> int {
-    if (!zip64 && value >= four_gib - margin) {
-      zip64 = true;
-      if (value >= max_size - margin) return 1;
-    }
-    return 0;
-  };
+  b2zip::ZipLayout L;
   std::vector<HeaderSpan> spans;
   std::vector<B2ZipCopy> copies;
-  struct Cat { u64 usize, csize, offset; u32 crc, time, ext_attr; u16 flag, method; };
-  std::vector<Cat> cat(n_entries);
-  u64 pos = 0;
   for (u32 i = 0; i < n_entries; i++) {
-    Cat &c = cat[i];
-    const u32 fl = flags ? flags[i] : 0;
-    c.flag = (fl & B2_ZIP_UNICODE_NAME) ? 0x0800 : 0;              // Language_Encoding_Flag_Bit (:222-224)
-    c.ext_attr = (fl & B2_ZIP_READ_ONLY) ? 1u : 0u;                // (:228-230)
-    c.time = dos_times ? dos_times[i] : 16789u * 65536u;           // Zip_Streams.default_time
-    c.usize = sizes[i];
-    c.crc = crc[i];
-    if (check_size(sizes[i])) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
-    c.offset = pos;
-    // decided BEFORE compression, with compressed_size = uncompressed_size (:233-243)
-    const bool ext = sizes[i] >= 0xFFFFFFFFull || c.offset >= 0xFFFFFFFFull;
+    u64 offset = 0, hbytes = 0;
+    if (!L.open_entry(sizes[i], nm[i].size(), &offset, &hbytes)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
     // Compression_inefficient <=> the stream is not smaller than the input (zip-compress.adb:468-490) -> Store (:224-237)
     const bool stored = streams[i].out_len >= sizes[i];
-    c.method = stored ? 0 : 12;
-    c.csize = stored ? sizes[i] : streams[i].out_len;
-    ByteSink h;
-    h.sig(3, 4);
-    h.u16le(10); h.u16le(c.flag); h.u16le(c.method); h.u32le(c.time); h.u32le(c.crc);
-    if (ext) { h.u32le(0xFFFFFFFFu); h.u32le(0xFFFFFFFFu); } else { h.u32le(c.csize); h.u32le(c.usize); }
-    h.u16le((u32)nm[i].size()); h.u16le(ext ? 20 : 0);
-    h.str(nm[i]);
-    if (ext) { h.u16le(1); h.u16le(16); h.u64le(c.usize); h.u64le(c.csize); }
-    const u64 payload = pos + h.b.size();
-    spans.push_back(HeaderSpan{pos, std::move(h.b)});
+    const u64 csize = stored ? sizes[i] : streams[i].out_len;
+    HeaderSpan h{offset, {}};
+    L.close_entry(nm[i], sizes[i], csize, crc[i], dos_times ? dos_times[i] : b2zip::ZipLayout::default_time, flags ? flags[i] : 0,
+                  stored ? 0 : 12, h.bytes);
+    const u64 payload = offset + hbytes;
+    spans.push_back(std::move(h));
     const u64 src = stored ? in_offsets[i] : streams[i].out_off;
-    for (u64 o = 0; o < c.csize; o += 65536) copies.push_back(B2ZipCopy{src + o, payload + o, (u32)std::min<u64>(65536, c.csize - o), stored ? 1u : 0u});
-    pos = payload + c.csize;
-    if (info) { info[i].crc32 = c.crc; info[i].zip_type = c.method; info[i].reserved = 0; info[i].compressed_size = c.csize; info[i].local_header_offset = c.offset; }
+    for (u64 o = 0; o < csize; o += 65536) copies.push_back(B2ZipCopy{src + o, payload + o, (u32)std::min<u64>(65536, csize - o), stored ? 1u : 0u});
+    if (info) { info[i].crc32 = crc[i]; info[i].zip_type = stored ? 0 : 12; info[i].reserved = 0; info[i].compressed_size = csize; info[i].local_header_offset = offset; }
   }
   {
-    ByteSink d;
-    const u64 cd_offset = pos;
-    u64 cd_size = 0;
-    if (!zip64 && n_entries >= 65535u) zip64 = true;               // too many entries for Zip_32 (:680-685)
-    for (u32 i = 0; i < n_entries; i++) {
-      const Cat &c = cat[i];
-      const bool ext = c.csize >= 0xFFFFFFFFull || c.usize >= 0xFFFFFFFFull || c.offset >= 0xFFFFFFFFull;
-      if (ext) zip64 = true;
-      d.sig(1, 2);
-      d.u16le(23); d.u16le(10); d.u16le(c.flag); d.u16le(c.method); d.u32le(c.time); d.u32le(c.crc);
-      d.u32le(ext ? 0xFFFFFFFFull : c.csize); d.u32le(ext ? 0xFFFFFFFFull : c.usize);
-      d.u16le((u32)nm[i].size()); d.u16le(ext ? 28 : 0);
-      d.u16le(0); d.u16le(0); d.u16le(0); d.u32le(c.ext_attr);
-      d.u32le(ext ? 0xFFFFFFFFull : c.offset);
-      d.str(nm[i]);
-      if (ext) { d.u16le(1); d.u16le(24); d.u64le(c.usize); d.u64le(c.csize); d.u64le(c.offset); }
-      cd_size += 46 + nm[i].size() + (ext ? 28 : 0);
-    }
-    if (n_entries) { if (check_size(cd_offset + cd_size + 1)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large"); }
-    u64 tot = n_entries, dtot = n_entries, cds = cd_size, cdo = cd_offset;
-    if (zip64) {
-      d.sig(6, 6);
-      d.u64le(44); d.u16le(0x2D); d.u16le(0x2D); d.u32le(0); d.u32le(0); d.u64le(n_entries); d.u64le(n_entries); d.u64le(cd_size); d.u64le(cd_offset);
-      d.sig(6, 7);
-      d.u32le(0); d.u64le(cd_offset + cd_size); d.u32le(1);
-      tot = dtot = 0xFFFF; cds = 0xFFFFFFFFull; cdo = 0xFFFFFFFFull;
-    }
-    d.sig(5, 6);
-    d.u16le(0); d.u16le(0); d.u16le((u32)dtot); d.u16le((u32)tot); d.u32le(cds); d.u32le(cdo); d.u16le(0);
-    const u64 n = d.b.size();
-    spans.push_back(HeaderSpan{pos, std::move(d.b)});
-    pos += n;
+    HeaderSpan d{L.pos, {}};
+    if (!L.finish(d.bytes)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
+    spans.push_back(std::move(d));
   }
+  const u64 pos = L.pos;
   *out_len = pos;
   if (pos > out_cap) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "output buffer too small");
   if (!out) B2_FAIL(B2_ERR_ARGUMENT, "out is NULL");
@@ -1905,6 +1873,251 @@ int b2_zip_create(b2_encoder *e, uint32_t n_entries, const uint8_t *in, const ui
   B2_CUDA_CHECK(cudaStreamSynchronize(e->st));
   for (const HeaderSpan &sp : spans) memcpy(out + sp.dst, sp.bytes.data(), sp.bytes.size());
   if (e->timing) { float ms = 0; cudaEventElapsedTime(&ms, e->ev_call[0], e->ev_call[1]); e->stats.call_ms += ms; }
+  return 0;
+}
+
+}  // extern "C"
+
+// ---- one archive written entry by entry (b2_zip_begin / add / finish, DESIGN.md §7c) ------------------------------------
+// Entries of at most W bytes are queued in stream.buf[0] and encoded together as one batch of b2_zip_create when the
+// next one would not fit.  A larger entry is one stream through the windows of b2_stream_* (size_hint = its size),
+// written behind its local header, whose length is known before compression; its Zip CRC-32 is folded window by window.
+namespace {
+// Progress of the archive: `done` counts on from the archive's bytes encoded before the call, the total is what was added.
+struct ProgressScope {
+  b2_encoder *e;
+  ProgressShim ps;
+  ProgressScope(b2_encoder *e_, u64 done0, u64 total) : e(e_), ps{e_->progress, e_->progress_user, done0, total} {
+    if (ps.fn) { e->progress = progress_shim; e->progress_user = &ps; }
+  }
+  ~ProgressScope() { e->progress = ps.fn; e->progress_user = ps.user; }
+};
+
+// Entries per batch of the queue.  Every queued entry costs device memory whatever its size: its chunk's two cut lists
+// (18 KiB at level 9), its output region (at least 5 KiB) and up to six blocks of batch workspace (about 330 KiB each,
+// DESIGN.md §3).  One entry per 32 KiB of W keeps that part of a batch below 64 bytes per byte of W.
+u64 zip_queue_max(u64 window) { return std::max<u64>(32, window >> 15); }
+
+void zip_close(b2_encoder *e) {
+  cudaStreamSynchronize(e->cst);                       // no upload may read the caller's `in` after the call returns
+  ZipState &Z = e->zip;
+  Z.open = false;
+  Z.layout = b2zip::ZipLayout();
+  Z.names.clear(); Z.queue.clear();
+  e->shard.open = e->shard.cut = e->shard.encoded = false;
+}
+
+// Encodes the queued entries as one batch and writes their archive bytes (local headers and payloads) to out[0 ..).
+int zip_flush(b2_encoder *e, u8 *out) {
+  ZipState &Z = e->zip;
+  const u32 nq = (u32)Z.queue.size();
+  if (!nq) return 0;
+  cudaStream_t st = e->st;
+  u8 *d = e->stream.buf[0];
+  B2_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_up, 0));
+  B2_CUDA_CHECK(cudaMemsetAsync(d + Z.q_end, 0, 128, st));
+  std::vector<u64> offs(nq), sizes(nq);
+  for (u32 i = 0; i < nq; i++) { offs[i] = Z.queue[i].off; sizes[i] = Z.queue[i].n; }
+  B2_TRY(zip_crc_device(e, d, nq, offs.data(), sizes.data()));
+  std::vector<u32> crc(nq);
+  B2_CUDA_CHECK(cudaMemcpyAsync(crc.data(), e->d_zcrc.p, nq * sizeof(u32), cudaMemcpyDeviceToHost, st));
+  std::vector<StreamDesc> streams(nq);
+  for (u32 i = 0; i < nq; i++) streams[i] = StreamDesc{offs[i], sizes[i], (i64)sizes[i], 0, 0, 0, 0};
+  {
+    ProgressScope ps(e, Z.done, Z.added);
+    B2_TRY(encode_streams(e, d, streams));
+  }
+  B2_CUDA_CHECK(cudaStreamSynchronize(st));
+  b2zip::ZipLayout &L = Z.layout;
+  const u64 base = L.pos;
+  std::vector<HeaderSpan> spans;
+  std::vector<B2ZipCopy> copies;
+  for (u32 i = 0; i < nq; i++) {
+    const ZipQueued &q = Z.queue[i];
+    u64 offset = 0, hbytes = 0;
+    if (!L.open_entry(q.n, q.name.size(), &offset, &hbytes)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
+    const bool stored = streams[i].out_len >= q.n;       // Store fallback, as in b2_zip_create
+    const u64 csize = stored ? q.n : streams[i].out_len;
+    HeaderSpan h{offset - base, {}};
+    L.close_entry(q.name, q.n, csize, crc[i], q.time, q.flags, stored ? 0 : 12, h.bytes);
+    const u64 payload = offset - base + hbytes;
+    spans.push_back(std::move(h));
+    const u64 src = stored ? q.off : streams[i].out_off;
+    for (u64 o = 0; o < csize; o += 65536) copies.push_back(B2ZipCopy{src + o, payload + o, (u32)std::min<u64>(65536, csize - o), stored ? 1u : 0u});
+  }
+  if (!copies.empty()) {
+    B2_TRY(e->d_zcopies.ensure(copies.size()));
+    B2_TRY(e->d_packed.ensure(L.pos - base + 64));
+    B2_CUDA_CHECK(cudaMemcpyAsync(e->d_zcopies.p, copies.data(), copies.size() * sizeof(B2ZipCopy), cudaMemcpyHostToDevice, st));
+    B2_TRY(b2k_zip_gather(st, e->d_zcopies.p, (u32)copies.size(), (const u8 *)e->d_out.p, d, e->d_packed.p));
+    e->launches_other += 1;
+    const u64 first = copies.front().dst_off, last = copies.back().dst_off + copies.back().len;
+    B2_CUDA_CHECK(cudaMemcpyAsync(out + first, e->d_packed.p + first, last - first, cudaMemcpyDeviceToHost, st));
+  }
+  B2_CUDA_CHECK(cudaStreamSynchronize(st));
+  for (const HeaderSpan &sp : spans) memcpy(out + sp.dst, sp.bytes.data(), sp.bytes.size());
+  Z.done += Z.q_bytes;
+  Z.queue.clear();
+  Z.q_end = Z.q_bytes = Z.q_bound = 0;
+  return 0;
+}
+
+// One entry above W: its local header and payload to out[0 ..), the stream written through the windows of b2_stream_*.
+int zip_add_windowed(b2_encoder *e, const std::string &name, u32 time, u32 flags, const u8 *in, u64 n, u8 *out, u64 out_cap) {
+  ZipState &Z = e->zip;
+  StreamState &S = e->stream;
+  b2zip::ZipLayout &L = Z.layout;
+  u64 offset = 0, hbytes = 0;
+  if (!L.open_entry(n, name.size(), &offset, &hbytes)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
+  u8 *payload = out + hbytes;
+  const u64 cap = out_cap - hbytes;
+  stream_reset(e, (i64)n);
+  u32 crc = 0;
+  u64 crc_done = 0;                                    // entry bytes folded into crc
+  auto crc_window = [&]() -> int {                     // the window's bytes that no window before it held
+    const u64 k = S.base + S.held - crc_done;
+    if (!k) return 0;
+    B2_CUDA_CHECK(cudaStreamWaitEvent(e->st, e->ev_up, 0));
+    const u64 at = crc_done - S.base;                  // an offset, not a pointer: k_zipcrc_tiles's vector loads need an aligned base
+    B2_TRY(zip_crc_device(e, S.buf[S.cur], 1, &at, &k));
+    u32 c = 0;
+    B2_CUDA_CHECK(cudaMemcpy(&c, e->d_zcrc.p, sizeof c, cudaMemcpyDeviceToHost));
+    crc = b2zip::crc32_combine(crc, c, k);
+    crc_done += k;
+    return 0;
+  };
+  ProgressScope ps(e, Z.done, Z.added);
+  const u64 full = S.window + S.margin;
+  u64 taken = 0;
+  for (;;) {                                           // b2_stream_write of the whole entry
+    const u64 k = std::min<u64>(full - S.held, n - taken);
+    B2_TRY(stream_upload(e, S.cur, S.held, in + taken, k));
+    S.held += k; taken += k;
+    if (S.held < full) break;
+    B2_TRY(crc_window());
+    B2_TRY(stream_window(e, false, in, n, &taken, payload, cap, 0));
+  }
+  B2_TRY(crc_window());
+  B2_TRY(stream_window(e, true, nullptr, 0, &taken, payload, cap, 0));   // b2_stream_end
+  if (taken != n || crc_done != n) B2_FAIL(B2_ERR_INTERNAL, "entry not taken whole");
+  const bool stored = S.out_end >= n;                  // Store fallback: the bytes from the caller's `in`
+  if (stored && n) memcpy(payload, in, n);
+  std::vector<u8> hdr;
+  L.close_entry(name, n, stored ? n : S.out_end, crc, time, flags, stored ? 0 : 12, hdr);
+  if (hdr.size() != hbytes) B2_FAIL(B2_ERR_INTERNAL, "local header length changed");
+  memcpy(out, hdr.data(), hbytes);
+  Z.done += n;
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int b2_zip_begin(b2_encoder *e, int duplicates, uint64_t window_bytes) {
+  if (!e) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  ZipState &Z = e->zip;
+  if (Z.open) B2_FAIL(B2_ERR_ARGUMENT, "an archive is already open on this handle");
+  if (e->stream.open) B2_FAIL(B2_ERR_ARGUMENT, "a stream is open on this handle (b2_stream_begin)");
+  if (duplicates != B2_ZIP_ADMIT_DUPLICATES && duplicates != B2_ZIP_ERROR_ON_DUPLICATE) B2_FAIL(B2_ERR_ARGUMENT, "bad duplicate policy");
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  B2_TRY(stream_buffers(e, window_bytes));
+  Z.layout = b2zip::ZipLayout();
+  Z.names.clear(); Z.queue.clear();
+  Z.q_end = Z.q_bytes = Z.q_bound = Z.cd_bound = Z.done = Z.added = 0;
+  Z.duplicates = duplicates;
+  Z.open = true;
+  return 0;
+}
+
+uint64_t b2_zip_add_bound(b2_encoder *e, uint64_t n, uint32_t name_bytes) {
+  const bool queued = e && e->zip.open && n <= e->stream.window;
+  const u64 q = e && e->zip.open ? e->zip.q_bound : 0;
+  return q + b2zip::ZipLayout::local_header_bytes(name_bytes, true) + (queued ? n : b2_stream_bound(nullptr, n));
+}
+
+uint64_t b2_zip_finish_bound(b2_encoder *e) {
+  if (!e || !e->zip.open) return b2zip::ZipLayout::end_records_max;
+  return e->zip.q_bound + e->zip.cd_bound + b2zip::ZipLayout::end_records_max;
+}
+
+int b2_zip_add(b2_encoder *e, const char *name, uint32_t name_bytes, uint32_t dos_time, uint32_t flags,
+               const uint8_t *in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
+  if (!e || !out_len || (n && !in) || (name_bytes && !name) || !out) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  ZipState &Z = e->zip;
+  if (!Z.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_zip_add without b2_zip_begin");
+  *out_len = 0;
+  if (name_bytes > 65535u) B2_FAIL(B2_ERR_ARGUMENT, "bad entry name length");
+  if (out_cap < b2_zip_add_bound(e, n, name_bytes)) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "output buffer below b2_zip_add_bound");
+  const std::string nm = b2zip::unixify(name, name_bytes);
+  if (Z.duplicates == B2_ZIP_ERROR_ON_DUPLICATE && Z.names.count(nm)) {   // Duplicate_name (zip-create.adb:138-147)
+    g_last_error = "Duplicate_name: Entry name = " + nm;
+    return B2_ERR_DUPLICATE_NAME;
+  }
+  const u64 out0 = Z.layout.pos;
+  auto run = [&]() -> int {
+    B2_CUDA_CHECK(cudaSetDevice(e->device));
+    if (Z.duplicates == B2_ZIP_ERROR_ON_DUPLICATE) Z.names.insert(nm);
+    Z.added += n;
+    Z.cd_bound += b2zip::ZipLayout::central_header_max(nm.size());
+    const StreamState &S = e->stream;
+    if (n > S.window) {
+      B2_TRY(zip_flush(e, out));
+      const u64 at = Z.layout.pos - out0;
+      return zip_add_windowed(e, nm, dos_time, flags, in, n, out + at, out_cap - at);
+    }
+    u64 at = (Z.q_end + 15) & ~15ull;
+    if (!Z.queue.empty() && (Z.q_bytes + n > S.window || at + n + 128 > S.buf_bytes || Z.queue.size() >= zip_queue_max(S.window))) {
+      B2_TRY(zip_flush(e, out));
+      at = 0;
+    }
+    B2_TRY(stream_upload(e, 0, at, in, n));
+    Z.queue.push_back(ZipQueued{nm, at, n, dos_time, flags});
+    Z.q_end = at + n; Z.q_bytes += n;
+    Z.q_bound += b2zip::ZipLayout::local_header_bytes(nm.size(), true) + n;
+    return 0;
+  };
+  const int rc = run();
+  if (rc) { const std::string msg = g_last_error; zip_close(e); g_last_error = msg; return rc; }
+  B2_CUDA_CHECK(cudaStreamSynchronize(e->cst));          // the caller may reuse `in` once this returns
+  *out_len = Z.layout.pos - out0;
+  return 0;
+}
+
+int b2_zip_finish(b2_encoder *e, uint8_t *out, uint64_t out_cap, uint64_t *out_len, b2_zip_entry_info *info, uint64_t info_cap,
+                  uint64_t *n_entries) {
+  if (!e || !out_len || !out || (info_cap && !info)) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  ZipState &Z = e->zip;
+  if (!Z.open) B2_FAIL(B2_ERR_ARGUMENT, "b2_zip_finish without b2_zip_begin");
+  *out_len = 0;
+  if (n_entries) *n_entries = 0;
+  if (out_cap < b2_zip_finish_bound(e)) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "output buffer below b2_zip_finish_bound");
+  b2zip::ZipLayout &L = Z.layout;
+  const u64 out0 = L.pos;
+  auto run = [&]() -> int {
+    B2_CUDA_CHECK(cudaSetDevice(e->device));
+    B2_TRY(zip_flush(e, out));
+    std::vector<u8> tail;
+    const u64 at = L.pos - out0;
+    if (!L.finish(tail)) B2_FAIL(B2_ERR_ARGUMENT, "Zip_Capacity_Exceeded: archive too large");
+    memcpy(out + at, tail.data(), tail.size());
+    return 0;
+  };
+  const int rc = run();
+  if (rc) { const std::string msg = g_last_error; zip_close(e); g_last_error = msg; return rc; }
+  for (size_t i = 0; i < L.cat.size() && i < info_cap; i++) {
+    const b2zip::ZipEntryRecord &c = L.cat[i];
+    info[i].crc32 = c.crc; info[i].zip_type = c.method; info[i].reserved = 0; info[i].compressed_size = c.csize;
+    info[i].local_header_offset = c.offset;
+  }
+  if (n_entries) *n_entries = L.cat.size();
+  *out_len = L.pos - out0;
+  zip_close(e);
+  return 0;
+}
+
+int b2_zip_abort(b2_encoder *e) {
+  if (!e) return B2_ERR_ARGUMENT;
+  if (e->zip.open) zip_close(e);
   return 0;
 }
 

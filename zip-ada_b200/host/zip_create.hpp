@@ -3,12 +3,18 @@
 // the C ABI of include/b2gpu.h.  The reference compresses an entry inside every Add_* call
 // (zip-create.adb:253-265, serial per entry); here the Add_* calls only queue the entry and Finish
 // sends the whole catalogue through ONE b2_zip_create call, so that the blocks of all entries share
-// the device batches (SURVEY.md §8f row 1, "Add_Streams-style front end").  The archive bytes are the
-// ones the reference writes.  No CPU fallback: without the CUDA library every call throws.
+// the device batches (SURVEY.md §8f row 1, "Add_Streams-style front end").  Zip_Writer below keeps the
+// reference's shape instead: every Add_* goes to the device at once (b2_zip_add) and the archive file grows as
+// entries complete, so memory does not grow with the archive.  The archive bytes are the ones the reference
+// writes.  No CPU fallback: without the CUDA library every call throws.
 #pragma once
 #include <cstdint>
 #include <cstdio>
+#include <fcntl.h>
 #include <fstream>
+#include <sys/mman.h>
+#include <sys/stat.h>
+#include <unistd.h>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -116,6 +122,112 @@ class Zip_Create_Info {
   std::vector<uint64_t> offs_, sizes_;
   std::string names_;
   std::vector<uint32_t> name_offs_{0}, times_, flags_;
+  std::vector<b2_zip_entry_info> info_;
+};
+
+// Zip.Create as the reference runs it (zip-create.adb:194-297): every Add_* compresses its entry at once, through
+// b2_zip_add, and the archive file is written as entries complete.  Host memory holds one entry's input and its
+// output; device memory is bounded by the window (include/b2gpu.h, b2_zip_begin).  The bytes are those of
+// Zip_Create_Info for the same calls.
+class Zip_Writer {
+ public:
+  Zip_Writer() = default;
+  Zip_Writer(const Zip_Writer &) = delete;
+  Zip_Writer &operator=(const Zip_Writer &) = delete;
+  ~Zip_Writer() {
+    if (enc_) { b2_zip_abort(enc_); b2_destroy(enc_); }
+  }
+  // Create_Archive (zip-create.ads:72-77).  window_bytes: see b2_zip_begin (0 = 512 MiB).
+  void Create_Archive(const std::string &Archive_Name, Compression_Method Compress_Method = BZip2_3,
+                      Duplicate_name_policy Duplicates = admit_duplicates, int device = 0, uint64_t window_bytes = 0) {
+    if (enc_ && (method_ != Compress_Method || device_ != device)) { b2_zip_abort(enc_); b2_destroy(enc_); enc_ = nullptr; }
+    if (!enc_ && b2_create((int)Compress_Method, device, &enc_) != B2_OK) throw Zip_error(std::string("b2_create: ") + b2_last_error());
+    method_ = Compress_Method; device_ = device;
+    b2_zip_abort(enc_);
+    if (b2_zip_begin(enc_, (int)Duplicates, window_bytes) != B2_OK) throw Zip_error(std::string("b2_zip_begin: ") + b2_last_error());
+    file_.close();
+    file_.open(Archive_Name, std::ios::binary | std::ios::trunc);
+    if (!file_) { b2_zip_abort(enc_); throw Zip_error("Create_Archive: cannot write " + Archive_Name); }
+    n_ = 0;
+    info_.clear();
+    created_ = true;
+  }
+  bool Is_Created() const { return created_; }
+  // Add_String (zip-create.ads:139-146)
+  void Add_String(const std::string &Contents, const std::string &Name_in_archive, bool Name_UTF_8_encoded = false,
+                  Time Creation_time = default_creation_time) {
+    Add_Stream(reinterpret_cast<const uint8_t *>(Contents.data()), Contents.size(), Name_in_archive, Creation_time,
+               Name_UTF_8_encoded, false);
+  }
+  // Add_Stream (zip-create.ads:94-103), the stream being a memory buffer: compressed and written before it returns.
+  void Add_Stream(const uint8_t *bytes, uint64_t size, const std::string &Name, Time Modification_time = default_creation_time,
+                  bool Is_Unicode_Name = false, bool Is_Read_Only = false) {
+    require_created();
+    out_.resize(b2_zip_add_bound(enc_, size, (uint32_t)Name.size()));
+    uint64_t len = 0;
+    const uint32_t fl = (Is_Unicode_Name ? B2_ZIP_UNICODE_NAME : 0u) | (Is_Read_Only ? B2_ZIP_READ_ONLY : 0u);
+    const int rc = b2_zip_add(enc_, Name.data(), (uint32_t)Name.size(), Modification_time, fl, bytes, size, out_.data(),
+                              out_.size(), &len);
+    if (rc == B2_ERR_DUPLICATE_NAME) throw Duplicate_name(b2_last_error());     // the archive stays open
+    if (rc != B2_OK) { created_ = false; throw Zip_error(std::string("b2_zip_add: ") + b2_last_error()); }
+    n_++;
+    write(len);
+  }
+  // Add_File (zip-create.ads:124-135): the file is mapped, one file at a time.
+  void Add_File(const std::string &File_Name, const std::string &Name_in_archive = "", bool Delete_file_after = false,
+                bool Name_UTF_8_encoded = false, Time Modification_time = default_creation_time, bool Is_read_only = false) {
+    require_created();
+    const int fd = open(File_Name.c_str(), O_RDONLY);
+    if (fd < 0) throw Zip_error("Add_File: cannot open " + File_Name);
+    struct stat st;
+    if (fstat(fd, &st) != 0) { close(fd); throw Zip_error("Add_File: cannot stat " + File_Name); }
+    const uint64_t size = (uint64_t)st.st_size;
+    void *map = nullptr;
+    if (size) {
+      map = mmap(nullptr, size, PROT_READ, MAP_PRIVATE, fd, 0);
+      if (map == MAP_FAILED) { close(fd); throw Zip_error("Add_File: cannot map " + File_Name); }
+    }
+    close(fd);
+    struct Unmap { void *p; uint64_t n; ~Unmap() { if (p) munmap(p, n); } } unmap{map, size};
+    Add_Stream(static_cast<const uint8_t *>(map), size, Name_in_archive.empty() ? File_Name : Name_in_archive,
+               Modification_time, Name_UTF_8_encoded, Is_read_only);
+    if (Delete_file_after) std::remove(File_Name.c_str());
+  }
+  // Add_Empty_Folder (zip-create.ads:157-161): an empty entry whose name ends with '/'
+  void Add_Empty_Folder(const std::string &Folder_Name, bool Name_UTF_8_encoded = false) {
+    std::string n = Folder_Name;
+    if (n.empty() || (n.back() != '/' && n.back() != '\\')) n += '/';
+    Add_Stream(nullptr, 0, n, default_creation_time, Name_UTF_8_encoded, false);
+  }
+  // Finish (zip-create.ads:265): the queued entries, central directory and end records; closes the file.
+  void Finish() {
+    require_created();
+    created_ = false;
+    out_.resize(b2_zip_finish_bound(enc_));
+    info_.resize(n_);
+    uint64_t len = 0, n = 0;
+    if (b2_zip_finish(enc_, out_.data(), out_.size(), &len, info_.data(), info_.size(), &n) != B2_OK)
+      throw Zip_error(std::string("b2_zip_finish: ") + b2_last_error());
+    write(len);
+    file_.close();
+    if (!file_) throw Zip_error("Finish: cannot write the archive");
+  }
+  // Compressed_Size / Final_Method of every entry, after Finish
+  const std::vector<b2_zip_entry_info> &Entries() const { return info_; }
+
+ private:
+  void require_created() const { if (!created_) throw Zip_error("archive not created"); }
+  void write(uint64_t len) {
+    file_.write(reinterpret_cast<const char *>(out_.data()), (std::streamsize)len);
+    if (!file_) { b2_zip_abort(enc_); created_ = false; throw Zip_error("cannot write the archive"); }
+  }
+  b2_encoder *enc_ = nullptr;
+  Compression_Method method_ = BZip2_3;
+  int device_ = 0;
+  bool created_ = false;
+  std::ofstream file_;
+  std::vector<uint8_t> out_;
+  uint64_t n_ = 0;
   std::vector<b2_zip_entry_info> info_;
 };
 
