@@ -333,6 +333,15 @@ B2_API int b2_dbg_block(b2_encoder *enc, const uint8_t *raw, uint32_t len,
                  uint8_t *rle_out, uint8_t *bwt_out, uint16_t *mtf_out, uint8_t *sel_out,
                  uint8_t *lens_out, uint8_t *bits_out, uint64_t bits_cap, b2_block_info *info);
 
+/* Stage A7 alone (MTF_and_RLE_2, bzip2-encoding.adb:318-413) on given last columns, as one batch with the production
+ * layout, plan and kernels: column j is cols[col_offs[j] .. + lens[j]), 0 <= lens[j] <= level * 100 000, with in_use
+ * taken from its bytes.  Writes its MTF index bytes to idx_out[col_offs[j] .. + lens[j]), its symbols (RUN_A / RUN_B,
+ * index + 1, EOB) to mtf_out one block after the other (mtf_cap >= the sum of lens[j] + 2), and n_mtf[j], n_groups[j].
+ * The slot padding, the masks and the outputs are poisoned before the launch.  Tests only. */
+B2_API int b2_dbg_mtf(b2_encoder *enc, const uint8_t *cols, const uint64_t *col_offs, const uint32_t *lens,
+                      uint32_t n_cols, uint8_t *idx_out, uint16_t *mtf_out, uint64_t mtf_cap, uint32_t *n_mtf,
+                      uint32_t *n_groups);
+
 typedef struct b2_chunk_trace {
   uint64_t start;
   uint32_t len, dyn_capacity;

@@ -510,8 +510,8 @@ struct BlockEncoder {
     else bwt_fast(rle_1_data.data(), n, bwt_data.data(), bwt_index);
   }
 
-  // :318-413
-  void MTF_and_RLE_2() {
+  // :318-413.  idx_out (may be null): the MTF index of every position of bwt_data (the search result of :384-392).
+  void MTF_and_RLE_2(u8 *idx_out = nullptr) {
     u8 unseq_to_seq[256];
     normal_symbols_in_use = 0;                                           // :320-328
     for (int i = 0; i < 256; i++)
@@ -535,11 +535,12 @@ struct BlockEncoder {
     };
     u8 mtf_symbol[256];
     for (int i = 0; i < 256; i++) mtf_symbol[i] = (u8)i;
-    for (u8 bt : bwt_data) {                                             // :378-407
-      u8 bt_seq = unseq_to_seq[bt];
+    for (size_t k = 0; k < bwt_data.size(); k++) {                       // :378-407
+      u8 bt_seq = unseq_to_seq[bwt_data[k]];
       int idx = 0;
       for (int search = 0; search < 256; search++)
         if (mtf_symbol[search] == bt_seq) { idx = search; break; }
+      if (idx_out) idx_out[k] = (u8)idx;
       for (int i = idx; i >= 1; i--) mtf_symbol[i] = mtf_symbol[i - 1];
       mtf_symbol[0] = bt_seq;
       if (idx == 0) run++;
@@ -1081,7 +1082,7 @@ struct orc_chunk_trace {
   u64 bits[4];
 };
 
-int orc_version() { return 62; }
+int orc_version() { return 63; }
 
 // Whole stream: what `Encode (option, size_hint)` writes through Write_Byte.
 int orc_encode_stream(const u8 *in, u64 n, int level, i64 size_hint, int bwt_mode,
@@ -1357,6 +1358,20 @@ int orc_encode_block(const u8 *raw, u32 len, int level, int bwt_mode,
     info->max_len = (u32)t.max_len; info->sample_width = (u32)t.sample_width; info->cost = t.best_cost;
     info->constructs = (u32)t.constructs; info->bits = t.bits;
   }
+  return 0;
+}
+
+// MTF_and_RLE_2 of a given last column col[0..n) (in_use = the bytes of col): the symbols mtf_data(1..mtf_last) into
+// mtf_out (>= n + 2 u16) and the MTF index of every position into idx_out (may be null).
+int orc_mtf_rle2(const u8 *col, u32 n, u16 *mtf_out, u32 *n_mtf, u8 *idx_out) {
+  EncoderConfig cfg{9, 0};
+  BlockEncoder be(cfg);
+  for (int i = 0; i < 256; i++) be.in_use[i] = false;
+  for (u32 i = 0; i < n; i++) be.in_use[col[i]] = true;
+  be.bwt_data.assign(col, col + n);
+  be.MTF_and_RLE_2(idx_out);
+  memcpy(mtf_out, be.mtf_data.data(), be.mtf_data.size() * 2);
+  *n_mtf = (u32)be.mtf_last;
   return 0;
 }
 

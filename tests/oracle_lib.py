@@ -100,6 +100,19 @@ def bwt(data, mode=0):
     return out[:a.size], origin.value
 
 
+def mtf_rle2(col):
+    """The reference's MTF_and_RLE_2 (bzip2-encoding.adb:318-413: linear search and shift) of a given last column, with
+    in_use taken from its bytes.  Returns (symbols as uint16, including EOB; MTF index of every position as uint8)."""
+    a = _u8(col)
+    mtf = np.zeros(a.size + 2, np.uint16)
+    idx = np.zeros(max(a.size, 1), np.uint8)
+    n = C.c_uint32(0)
+    rc = lib().orc_mtf_rle2(a.ctypes.data_as(C.c_void_p), C.c_uint32(a.size), mtf.ctypes.data_as(C.c_void_p), C.byref(n),
+                            idx.ctypes.data_as(C.c_void_p))
+    assert rc == 0, rc
+    return mtf[:n.value].copy(), idx[:a.size].copy()
+
+
 def segment(data, profile):
     a = _u8(data)
     cuts = np.zeros(4096, np.uint32)

@@ -64,7 +64,7 @@ EXPORTS = ["b2_create", "b2_destroy", "b2_bound", "b2_encode_stream", "b2_encode
            "b2_shard_margin", "b2_shard_plan", "b2_shard_open", "b2_shard_cut", "b2_shard_encode", "b2_shard_resolve",
            "b2_shard_finish", "b2_encode_stream_multi", "b2_set_progress", "b2_verify_stream",
            "b2_stream_begin", "b2_stream_bound", "b2_stream_write", "b2_stream_end", "b2_stream_abort", "b2_dbg_segment",
-           "b2_zip_begin", "b2_zip_add_bound", "b2_zip_add", "b2_zip_finish_bound", "b2_zip_finish", "b2_zip_abort"]
+           "b2_zip_begin", "b2_zip_add_bound", "b2_zip_add", "b2_zip_finish_bound", "b2_zip_finish", "b2_zip_abort", "b2_dbg_mtf"]
 
 _lib = None
 
@@ -112,6 +112,8 @@ def lib():
         _lib.b2_get_segments.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
         _lib.b2_dbg_segment.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p,
                                         C.POINTER(C.c_uint32), C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]
+        _lib.b2_dbg_mtf.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
+                                    C.c_uint64, C.c_void_p, C.c_void_p]
         _lib.b2_set_progress.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         _lib.b2_verify_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_int, C.c_uint64, C.POINTER(VerifyResult)]
         _lib.b2_shard_margin.restype = C.c_uint64
@@ -377,6 +379,30 @@ class Encoder:
                                     C.byref(n1), cuts.shape[1], series.ctypes.data, series.size, paths.ctypes.data))
         steps = a.size - 16_000 if a.size > 20_000 else 0
         return dict(cuts=[cuts[0, :n0.value].copy(), cuts[1, :n1.value].copy()], series=series[:steps].copy(), paths=paths)
+
+    def dbg_mtf(self, cols):
+        """Stage A7 alone on the given last columns (one batch, production plan and kernels): one dict per column with
+        idx (uint8 MTF index of every position), mtf (uint16 symbols), n_mtf and n_groups."""
+        arrs = [_u8(c) for c in cols]
+        lens = np.array([a.size for a in arrs], np.uint32)
+        offs = np.zeros(len(arrs), np.uint64)
+        if len(arrs) > 1:
+            offs[1:] = np.cumsum(lens[:-1].astype(np.uint64))
+        flat = np.concatenate(arrs) if arrs else np.zeros(0, np.uint8)
+        flat = flat if flat.size else np.zeros(1, np.uint8)
+        idx = np.zeros(max(int(lens.sum()), 1), np.uint8)
+        cap = int(lens.sum()) + 2 * len(arrs)
+        mtf = np.zeros(max(cap, 1), np.uint16)
+        n_mtf = np.zeros(max(len(arrs), 1), np.uint32)
+        n_groups = np.zeros(max(len(arrs), 1), np.uint32)
+        _check(lib().b2_dbg_mtf(self._h, flat.ctypes.data, offs.ctypes.data, lens.ctypes.data, len(arrs), idx.ctypes.data,
+                                mtf.ctypes.data, cap, n_mtf.ctypes.data, n_groups.ctypes.data))
+        out, mo = [], 0
+        for j in range(len(arrs)):
+            o, n, m = int(offs[j]), int(lens[j]), int(n_mtf[j])
+            out.append(dict(idx=idx[o:o + n].copy(), mtf=mtf[mo:mo + m].copy(), n_mtf=m, n_groups=int(n_groups[j])))
+            mo += m
+        return out
 
     def dbg_block(self, data):
         a = _u8(data)

@@ -316,6 +316,42 @@ u64 layout_jobs(std::vector<B2Job> &jobs, int level) {
   return pos;
 }
 
+// The MTF stage's plan (host; needs n and n_used of every block): the 4096-position tiles of k_mtf_masks (b.tile0 = a
+// block's first) and the segments of B2_MTF_SEG positions, blocks with <= 64 bytes in use first, then <= 128, then
+// the others (the kernel classes of b2k_mtf).
+struct MtfPlan {
+  std::vector<B2SortTile> tiles, segs;
+  u32 n_small = 0, n_mid = 0;
+};
+
+void plan_mtf(std::vector<B2Job> &jobs, MtfPlan &P) {
+  std::vector<B2SortTile> mid, big;
+  P.tiles.clear(); P.segs.clear();
+  for (u32 j = 0; j < (u32)jobs.size(); j++) {
+    B2Job &b = jobs[j];
+    b.tile0 = (u32)P.tiles.size();
+    for (u32 s = 0; s < b.n; s += B2_MTF_TILE) P.tiles.push_back(B2SortTile{j, s});
+    for (u32 s = 0; s < b.n; s += B2_MTF_SEG) (b.n_used <= 64 ? P.segs : b.n_used <= 128 ? mid : big).push_back(B2SortTile{j, s});
+  }
+  P.n_small = (u32)P.segs.size(); P.n_mid = (u32)mid.size();
+  P.segs.insert(P.segs.end(), mid.begin(), mid.end());
+  P.segs.insert(P.segs.end(), big.begin(), big.end());
+}
+
+// Uploads the plan and launches the stage on w's stream: w->d_bwt (the last columns) -> w->d_idx, w->d_mtf and
+// n_mtf / n_groups of w->d_jobs.
+int launch_mtf(Workspace *w, u32 J, const MtfPlan &P) {
+  cudaStream_t st = w->st;
+  if (!P.tiles.empty())
+    B2_CUDA_CHECK(cudaMemcpyAsync(w->d_mtiles.p, P.tiles.data(), P.tiles.size() * sizeof(B2SortTile), cudaMemcpyHostToDevice, st));
+  if (!P.segs.empty())
+    B2_CUDA_CHECK(cudaMemcpyAsync(w->d_msegs.p, P.segs.data(), P.segs.size() * sizeof(B2SortTile), cudaMemcpyHostToDevice, st));
+  B2_TRY(b2k_mtf(st, w->d_jobs.p, J, w->d_mtiles.p, (u32)P.tiles.size(), w->d_msegs.p, P.n_small, P.n_mid, (u32)P.segs.size(), w->d_bwt.p,
+                 w->d_m16.p, w->d_m256.p, w->d_tilemask.p, w->d_idx.p, w->d_mtf.p));
+  w->launches += 4;
+  return 0;
+}
+
 // Runs one batch through RLE1 -> BWT -> MTF/RLE2 -> entropy search -> bit packing on workspace w.
 // On return w->batch_jobs holds the device's view of the jobs (n, crc, origin, nbits, bits_off ...).
 int run_batch(b2_encoder *e, Workspace *w, const u8 *d_in, std::vector<B2Job> &jobs) {
@@ -337,7 +373,6 @@ int run_batch(b2_encoder *e, Workspace *w, const u8 *d_in, std::vector<B2Job> &j
   // group arena offsets need n (M <= n + 1)
   u32 gpos = 0, max_g = 1;
   std::vector<u32> ids(J), ns(J);
-  std::vector<B2SortTile> mtiles, msegs, msegs_mid, msegs_big;
   for (u32 j = 0; j < J; j++) {
     B2Job &b = w->batch_jobs[j];
     if (b.n > b.cap) B2_FAIL(B2_ERR_INTERNAL, "RLE1 output exceeds its slot");
@@ -346,11 +381,10 @@ int run_batch(b2_encoder *e, Workspace *w, const u8 *d_in, std::vector<B2Job> &j
     max_g = std::max(max_g, gmax);
     ids[j] = j; ns[j] = b.n;
     b.na = b.n;
-    b.tile0 = (u32)mtiles.size();
-    for (u32 s = 0; s < b.n; s += B2_MTF_TILE) mtiles.push_back(B2SortTile{j, s});
-    for (u32 s = 0; s < b.n; s += B2_MTF_SEG) (b.n_used <= 64 ? msegs : b.n_used <= 128 ? msegs_mid : msegs_big).push_back(B2SortTile{j, s});
     w->block_bytes += b.n;
   }
+  MtfPlan mplan;
+  plan_mtf(w->batch_jobs, mplan);
   w->blocks += J;
   w->total_groups = gpos;
   // write grp_off / tile0 / na back (the only fields changed on the host)
@@ -381,16 +415,7 @@ int run_batch(b2_encoder *e, Workspace *w, const u8 *d_in, std::vector<B2Job> &j
   }
   {
     StageTimer tm(e, st, w->ev, &w->stage_ms[3]);
-    if (!mtiles.empty())
-      B2_CUDA_CHECK(cudaMemcpyAsync(w->d_mtiles.p, mtiles.data(), mtiles.size() * sizeof(B2SortTile), cudaMemcpyHostToDevice, st));
-    const u32 n_small = (u32)msegs.size(), n_mid = (u32)msegs_mid.size();
-    msegs.insert(msegs.end(), msegs_mid.begin(), msegs_mid.end());
-    msegs.insert(msegs.end(), msegs_big.begin(), msegs_big.end());
-    if (!msegs.empty())
-      B2_CUDA_CHECK(cudaMemcpyAsync(w->d_msegs.p, msegs.data(), msegs.size() * sizeof(B2SortTile), cudaMemcpyHostToDevice, st));
-    B2_TRY(b2k_mtf(st, w->d_jobs.p, J, w->d_mtiles.p, (u32)mtiles.size(), w->d_msegs.p, n_small, n_mid, (u32)msegs.size(), w->d_bwt.p, w->d_m16.p,
-                   w->d_m256.p, w->d_tilemask.p, w->d_idx.p, w->d_mtf.p));
-    w->launches += 4;
+    B2_TRY(launch_mtf(w, J, mplan));
   }
   // exact group counts: the ranking heap sorts size their shared memory by the largest block
   B2_CUDA_CHECK(cudaMemcpyAsync(w->batch_jobs.data(), w->d_jobs.p, J * sizeof(B2Job), cudaMemcpyDeviceToHost, st));
@@ -2193,6 +2218,60 @@ int b2_dbg_block(b2_encoder *e, const uint8_t *raw, uint32_t len, uint8_t *rle_o
     info->n_used = b.n_used; info->n_sel = b.n_groups; info->ec_count = (u32)ec; info->max_len = (u32)max_len;
     info->sample_width = (u32)sw; info->cost = b.best_cost; info->pad = 0; info->bits = b.nbits;
   }
+  return 0;
+}
+
+int b2_dbg_mtf(b2_encoder *e, const uint8_t *cols, const uint64_t *col_offs, const uint32_t *lens, uint32_t n_cols,
+               uint8_t *idx_out, uint16_t *mtf_out, uint64_t mtf_cap, uint32_t *n_mtf, uint32_t *n_groups) {
+  if (!e || n_cols == 0 || n_cols > e->batch_jobs_max || !col_offs || !lens || !idx_out || !mtf_out || !n_mtf || !n_groups)
+    B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+  u64 need = 0;
+  for (u32 j = 0; j < n_cols; j++) {
+    if (lens[j] > (u32)e->level * 100000u) B2_FAIL(B2_ERR_ARGUMENT, "column longer than a block of this level");
+    if (lens[j] && !cols) B2_FAIL(B2_ERR_ARGUMENT, "bad argument");
+    need += (u64)lens[j] + 2;
+  }
+  if (mtf_cap < need) B2_FAIL(B2_ERR_OUTPUT_TOO_SMALL, "mtf_out too small");
+  B2_NO_STREAM(e);
+  B2_CUDA_CHECK(cudaSetDevice(e->device));
+  Workspace *w = e->ws[0];
+  cudaStream_t st = w->st;
+  std::vector<B2Job> jobs(n_cols);
+  for (u32 j = 0; j < n_cols; j++) {
+    B2Job &b = jobs[j];
+    memset(&b, 0, sizeof b);
+    b.raw_len = b.n = lens[j];
+    const uint8_t *c = cols + col_offs[j];
+    for (u32 i = 0; i < b.n; i++) b.in_use[c[i] >> 5] |= 1u << (c[i] & 31);
+    for (int q = 0; q < 8; q++) b.n_used += (u32)__builtin_popcount(b.in_use[q]);
+  }
+  const u64 T = layout_jobs(jobs, e->level);
+  B2_TRY(ensure_batch_workspace(w, (size_t)T + 64, n_cols));
+  // Poison: slot padding and index bytes 0xA5, symbols 0xA5A5, masks 0 (an unwritten mask reads as "no byte here", so
+  // the list rebuild misses bytes).  A read of anything not written, or an output not written, shows as a difference.
+  B2_CUDA_CHECK(cudaMemsetAsync(w->d_bwt.p, 0xA5, w->d_bwt.cap, st));
+  B2_CUDA_CHECK(cudaMemsetAsync(w->d_idx.p, 0xA5, w->d_idx.cap, st));
+  B2_CUDA_CHECK(cudaMemsetAsync(w->d_m16.p, 0, w->d_m16.cap * sizeof(u32), st));
+  B2_CUDA_CHECK(cudaMemsetAsync(w->d_m256.p, 0, w->d_m256.cap * sizeof(u32), st));
+  B2_CUDA_CHECK(cudaMemsetAsync(w->d_mtf.p, 0xA5, w->d_mtf.cap * sizeof(u16), st));
+  for (u32 j = 0; j < n_cols; j++)
+    if (jobs[j].n) B2_CUDA_CHECK(cudaMemcpyAsync(w->d_bwt.p + jobs[j].pos_off, cols + col_offs[j], jobs[j].n, cudaMemcpyHostToDevice, st));
+  MtfPlan P;
+  plan_mtf(jobs, P);
+  B2_CUDA_CHECK(cudaMemcpyAsync(w->d_jobs.p, jobs.data(), n_cols * sizeof(B2Job), cudaMemcpyHostToDevice, st));
+  B2_TRY(launch_mtf(w, n_cols, P));
+  B2_CUDA_CHECK(cudaMemcpyAsync(jobs.data(), w->d_jobs.p, n_cols * sizeof(B2Job), cudaMemcpyDeviceToHost, st));
+  B2_CUDA_CHECK(cudaStreamSynchronize(st));
+  u64 mo = 0;
+  for (u32 j = 0; j < n_cols; j++) {
+    const B2Job &b = jobs[j];
+    if (b.n_mtf > b.n + 2) B2_FAIL(B2_ERR_INTERNAL, "more symbols than positions");
+    if (b.n) B2_CUDA_CHECK(cudaMemcpyAsync(idx_out + col_offs[j], w->d_idx.p + b.pos_off, b.n, cudaMemcpyDeviceToHost, st));
+    B2_CUDA_CHECK(cudaMemcpyAsync(mtf_out + mo, w->d_mtf.p + b.mtf_off, (size_t)b.n_mtf * sizeof(u16), cudaMemcpyDeviceToHost, st));
+    n_mtf[j] = b.n_mtf; n_groups[j] = b.n_groups;
+    mo += b.n_mtf;
+  }
+  B2_CUDA_CHECK(cudaStreamSynchronize(st));
   return 0;
 }
 

@@ -56,7 +56,9 @@ __host__ __device__ inline void b2_triple(int level, int t, int &max_len, int &s
 #define B2_CUDA_CHECK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { b2_set_error(__FILE__, __LINE__, cudaGetErrorString(e_)); return 10; } } while (0)
 void b2_set_error(const char *file, int line, const char *msg);
 
-#ifdef __CUDACC__
+// Device helpers; the host emulation of tests/emu compiles them too, against its restated intrinsics (cuda_emu.h defines
+// B2_EMU_DEVICE_HELPERS).
+#if defined(__CUDACC__) || defined(B2_EMU_DEVICE_HELPERS)
 __device__ __forceinline__ u32 lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ u32 warp_id() { return threadIdx.x >> 5; }
 
